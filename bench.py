@@ -132,6 +132,24 @@ def encoder_algorithmic_bytes(reads, regions, n_out: int, out_bytes: int) -> int
     return rd + ref + n_out * out_bytes
 
 
+DUMP_BYTES = 60 * 10 ** 6          # the files stay under 64 MB with their headers
+
+
+def dump_outputs(d: str, arrays: dict, n: int) -> None:
+    """--dump-outputs: arrays with one row per output record / image, as d/<name>.npy (float32 where that is exact, else
+    float64).  All n rows when they fit in DUMP_BYTES, else a sample drawn with a fixed seed (the same rows for the same n);
+    sample_rows.npy holds the row indices and n_rows.npy the row count."""
+    exact32 = lambda a: a.dtype == np.float32 or (a.dtype.kind in "iu" and a.dtype.itemsize <= 2)      # noqa: E731
+    row_bytes = sum((4 if exact32(a) else 8) * int(np.prod(a.shape[1:])) for a in arrays.values()) + 8
+    keep = DUMP_BYTES // row_bytes
+    rows = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "sample_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(d, "n_rows.npy"), np.array([n], dtype=np.float64))
+    for k, a in arrays.items():
+        np.save(os.path.join(d, k + ".npy"), a[rows].astype(np.float32 if exact32(a) else np.float64))
+
+
 def platform_of(cfg):
     from pepper_b200 import synth
     plat = synth.ONT if cfg["platform"] == "ONT" else synth.HIFI
@@ -257,6 +275,11 @@ def run_variant(args, cfg):
     rstat, rall = rank_stats(mine, world, dev)
     counts = dvc.buffer.counts.cpu().numpy()
     n_job = int(counts.sum())
+    if args.dump_outputs and rank == 0:                     # the last timed step's records, as the writer rank receives them
+        rec = dvc.buffer.to_host()
+        dump_outputs(args.dump_outputs, {"probs": rec["probs"], "position": rec["position"], "region": rec["region"], "depth": rec["depth"],
+                                         "freq": rec["freq"], "key": np.ascontiguousarray(rec["key"]).view(np.uint8).reshape(-1, rec.dtype["key"].itemsize)},
+                     rec.shape[0])
 
     # ---- end-to-end leg: pinned host reads -> H2D -> kernels -> gather -> D2H of the job's records on the writer rank
     hr = HostReads(reads, pin=True)
@@ -654,6 +677,8 @@ def run_polish(args, cfg):
     e1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:                     # what the last timed step wrote into `out`
+        dump_outputs(args.dump_outputs, {k: v[:n_img].cpu().numpy() for k, v in out.items()}, n_img)
     ms = e0.elapsed_time(e1)
     if world > 1:
         tt = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -890,7 +915,12 @@ def main():
     ap.add_argument("--inflate-host-share", type=float, default=None,
                     help="from-files leg: share of the BGZF blocks inflated by the host pool beside the kernel (default 0: all on the GPU)")
     ap.add_argument("--host-inflate", action="store_true", help="from-files leg with the host zlib pool instead of the GPU inflate")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32 / float64, at most 64 MB: a seeded "
+                         "sample of the rows of a larger output)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     cfg = CONFIGS[args.config]
     if args.regions is None:
         args.regions = int(os.environ.get("PB_BENCH_REGIONS", cfg["regions"]))

@@ -10,14 +10,13 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from pepper_b200 import synth  # noqa: E402
 from oracle import oracle  # noqa: E402
 
-oracle.build()
-assert oracle.have_ref_getreads(), "needs /root/reference"
-
 SEED, CONTIG, COV, START = 31, 24000, 25, 5000
 QUERIES = [(START + 900, START + 2101, False, 0, 0), (START + 10000, START + 11201, False, 0, 0),
            (START - 100, START + 6101, True, 5, 7), (START + 23000, START + 26000, False, 0, 0)]
 
 if __name__ == "__main__":
+    oracle.build()
+    assert oracle.have_ref_getreads(), "needs oracle/_ref/libref_getreads.so, built from the reference sources"
     rec, _ = synth.simulate_contig_records(CONTIG, COV, synth.ONT, SEED, contig_start=START)
     out = {}
     for qi, (s, e, supp, mq, bq) in enumerate(QUERIES):

@@ -1,21 +1,23 @@
 """GPU parity at BASELINE.json's own sizes (VERDICT r1 item 1): full 100 kb intervals (+2 x 100 bp halo = 100,201
 positions per region, pepper_variant ImageGenerationUI.py:307-316) compared with the UNMODIFIED reference encoder
-compiled into oracle/_ref (falls back to the plain-C port when _ref is absent), for the ONT and HiFi presets, and one
-batch of 100 distinct regions through the public host-buffer call so that the region-group pipelining of
+compiled into oracle/_ref (through the digests of its outputs, tests/golden/refdigest.py) and with the plain-C port, for
+the ONT and HiFi presets, and one batch of 100 distinct regions through the public host-buffer call so that the region-group pipelining of
 pb_variant_call_host (first group 24, then 96 regions) and its capacity retry cross a group boundary.  Network outputs
 of the shipped (tcgen05) mode are compared with oracle/nets.py for the candidates of sampled regions."""
 import numpy as np
 import pytest
 
 from pepper_b200 import synth
+from tests.golden import refdigest
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-3
 MARGIN = 1e-4
 
 
-def _impl(oracle):
-    return "ref" if oracle.have_ref() else "port"
+def _fields(calls):
+    return dict(keys=calls.keys, positions=calls.positions, depths=calls.depths, freqs=calls.freqs, region_of=calls.region_of,
+                images_i8=calls.images)
 
 
 def _same_candidates(got, want, oracle, images=True):
@@ -42,8 +44,9 @@ def test_full_size_regions_vs_reference(oracle_built, platform, params, cov, see
     state = nets.make_variant_weights(seed)
     caller = VariantCaller(state)
     calls = caller.call(reads, regions, params, want_images=True)
-    want = oracle_built.variant_encode(reads, regions, params, _impl(oracle_built))
+    want = oracle_built.variant_encode(reads, regions, params, "port")
     _same_candidates(calls, want, oracle_built)
+    refdigest.expect("gpu_full_size_seed%d" % seed, _fields(calls))
     assert len(calls) > (1000 if platform is synth.ONT else 100)
     probs = nets.variant_predict(state, calls.images, threads=16)
     assert np.abs(probs - calls.probs).max() < TOL, np.abs(probs - calls.probs).max()
@@ -64,12 +67,11 @@ def test_100_full_size_regions_cross_group_boundary(oracle_built):
     state = nets.make_variant_weights(3)
     caller = VariantCaller(state)
     calls = caller.call(reads, regions, params, want_images=True)
-    impl = _impl(oracle_built)
     # the oracle one region at a time (that is how the reference runs: one RegionalSummaryGenerator per interval)
     off = 0
     for r in range(n_regions):
         sub, tab = synth.region_batch(reads, regions, r)
-        w = oracle_built.variant_encode(sub, tab, params, impl)
+        w = oracle_built.variant_encode(sub, tab, params, "port")
         n = len(w["keys"])
         sl = slice(off, off + n)
         assert calls.keys[off:off + n] == w["keys"], r
@@ -80,6 +82,7 @@ def test_100_full_size_regions_cross_group_boundary(oracle_built):
         assert np.array_equal(calls.images[sl], oracle_built.images_to_int8(w["images"])), r
         off += n
     assert off == len(calls) > 9472 * 3
+    refdigest.expect("gpu_full_size_100_regions_seed103", _fields(calls))
     # capacity far too small: the retry happens inside the second group and must give the same answer
     small = caller.call(reads, regions, params, capacity=40000)
     assert np.array_equal(small.probs, calls.probs) and np.array_equal(small.positions, calls.positions)

@@ -1,106 +1,57 @@
-"""CPU (needs /root/reference, i.e. runs in the build container): the four store layouts written by pepper_b200/datastore.py
-are read back by the reference's OWN reader code — pepper_variant dataloader_predict.SequenceDataset (a9),
-pepper dataloader_predict.SequenceDataset (a12), pepper Stitch.small_chunk_stitch (a14) and
-pepper_variant CandidateFinder.small_chunk_stitch (a16, which parses ``str(candidates[i])``) — through an `h5py` stand-in
-backed by the npz container (h5py / libhdf5 are in neither image).  The stand-in hands datasets back unchanged, so a wrong
-dtype (e.g. fixed bytes instead of str) breaks the reference's parsing exactly as it would under h5py 2.10."""
-import os
-import sys
-import types
+"""CPU: the four store layouts written by pepper_b200/datastore.py are the ones the reference's OWN reader code reads back —
+pepper_variant dataloader_predict.SequenceDataset (a9), pepper dataloader_predict.SequenceDataset (a12), pepper
+Stitch.small_chunk_stitch (a14) and pepper_variant CandidateFinder.small_chunk_stitch (a16, which parses
+``str(candidates[i])``).  tests/golden/make_golden_stores.py runs those readers on the stores written here, through an
+`h5py` stand-in backed by the npz container, and records digests of each store's layout and of what the reader returned
+(tests/golden/refdigest.py).  Each test writes its store again and checks that the layout (dataset paths, dtypes, shapes,
+contents) is the one the reader read, and that what the reader returned is what the inputs (or the oracle) say.  The
+stand-in hands datasets back unchanged, so a wrong dtype (e.g. fixed bytes instead of str) breaks the reference's parsing
+exactly as it would under h5py 2.10."""
 import numpy as np
-import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
+from pepper_b200 import datastore as ds
+from tests.golden import refdigest
 
-
-class _Leaf:
-    def __init__(self, a):
-        self.a = a
-
-    def __getitem__(self, k):
-        if k != ():
-            return self.a[k]
-        return self.a[()] if self.a.shape == () else self.a
+VARIANT_OPTIONS = dict(snp_p_value=0.1, insert_p_value=0.1, delete_p_value=0.1, snp_p_value_in_lc=0.3, insert_p_value_in_lc=0.35,
+                       delete_p_value_in_lc=0.25, report_snp_above_freq=0.0, report_indel_above_freq=0.6)
 
 
-class _Node:
-    def __init__(self, store, prefix):
-        self.s, self.p = store, prefix
-
-    def keys(self):
-        return self.s.keys(self.p) if self.p else sorted({k.split("/", 1)[0] for k in self.s.data})
-
-    def __contains__(self, k):
-        return k in self.keys()
-
-    def __getitem__(self, k):
-        path = (self.p + "/" + k).strip("/")
-        return _Leaf(self.s.data[path]) if path in self.s.data else _Node(self.s, path)
+def layout(fname):
+    """Dataset path, dtype, shape and content digest of every dataset of a store."""
+    d = ds._Store(fname, mode="r", backend="npz").data
+    return [[k, d[k].dtype.str, list(d[k].shape), refdigest.digest(d[k])] for k in sorted(d)]
 
 
-@pytest.fixture()
-def ref_modules(monkeypatch):
-    from pepper_b200 import datastore as ds
-
-    class _File(_Node):
-        def __init__(self, name, mode="r"):
-            super().__init__(ds._Store(name, mode="r", backend="npz"), "")
-
-        def __enter__(self):
-            return self
-
-        def __exit__(self, *a):
-            pass
-
-        def close(self):
-            pass
-    h5 = types.ModuleType("h5py"); h5.File = _File
-    tv = types.ModuleType("torchvision"); tvt = types.ModuleType("torchvision.transforms")
-    tvt.Compose = lambda x: x; tvt.ToTensor = lambda: None; tv.transforms = tvt
-    pv = types.ModuleType("pepper_variant.build.PEPPER_VARIANT")
-
-    class CandidateImagePrediction:
-        def __init__(self, contig, position, depth, candidates, candidate_frequency, prediction_base, prediction_type):
-            self.contig, self.position, self.depth = contig, position, depth
-            self.candidates, self.candidate_frequency = candidates, candidate_frequency
-            self.prediction_base, self.prediction_type = prediction_base, prediction_type
-    pv.CandidateImagePrediction = CandidateImagePrediction
-    bv = types.ModuleType("pepper_variant.build"); bv.PEPPER_VARIANT = pv
-    bp = types.ModuleType("pepper.build"); bp.PEPPER = types.ModuleType("pepper.build.PEPPER")
-    for name, mod in {"h5py": h5, "torchvision": tv, "torchvision.transforms": tvt, "pepper_variant.build": bv,
-                      "pepper_variant.build.PEPPER_VARIANT": pv, "pepper.build": bp, "pepper.build.PEPPER": bp.PEPPER}.items():
-        monkeypatch.setitem(sys.modules, name, mod)
-    monkeypatch.syspath_prepend(REF)
-    monkeypatch.setattr(np, "int", int, raising=False)
-    for m in [k for k in sys.modules if k.startswith(("pepper.modules", "pepper_variant.modules"))]:
-        monkeypatch.delitem(sys.modules, m)
-    return pv
+def _s(x):
+    """A str stays itself; anything else (e.g. bytes) shows its type."""
+    return x if isinstance(x, str) else repr(x)
 
 
-def test_variant_image_store_read_by_reference_dataloader(tmp_path, ref_modules):
-    from pepper_b200 import datastore as ds
-    from pepper_variant.modules.python.models.dataloader_predict import SequenceDataset
-    f = str(tmp_path / "img.hdf5")
+# ---- a9: variant image store -> pepper_variant dataloader_predict.SequenceDataset
+def write_variant_images(f):
+    """Writes the store; returns the (contig, position, depth, candidates, frequencies, image) items it must read back as."""
     rng = np.random.default_rng(1)
     imgs = rng.integers(-128, 128, size=(3, 33, 26)).astype(np.int8)
     keys = ["1T", "2ACG", "3" + "ACGT" * 15]
     with ds.VariantImageStore(f, backend="npz") as s:
         s.write_summary("chr20_1000_2000", "chr20", [1001, 1500, 1999], [30, 125, 7], keys, [5, 12, 3], imgs)
-    data = SequenceDataset(None, input_file=f)
-    assert len(data) == 3
-    for i in range(3):
-        contig, position, depth, candidate, freq, image = data[i]
-        assert contig == "chr20" and position == [1001, 1500, 1999][i] and depth == [30, 125, 7][i]
-        assert [str(c) for c in candidate] == [keys[i]] and isinstance(candidate[0], str)
-        assert list(freq) == [[5], [12], [3]][i] and np.array_equal(image, imgs[i]) and image.dtype == np.int8
-    batch = SequenceDataset.my_collate([data[0], data[1]])
-    assert tuple(batch[5].shape) == (2, 33, 26)
+    return [("chr20", p, d, [k], [fr], im) for p, d, k, fr, im in zip([1001, 1500, 1999], [30, 125, 7], keys, [5, 12, 3], imgs)]
 
 
-def test_variant_prediction_store_read_by_reference_candidate_finder(tmp_path, ref_modules):
-    from pepper_b200 import datastore as ds
-    from oracle import find_candidates as ofc
+def variant_items(items, collated_shape):
+    return [[_s(c), int(p), int(d), [_s(x) for x in cand], [int(x) for x in np.ravel(fr)], np.asarray(im).dtype.str,
+             np.asarray(im).astype(np.int64).tolist()] for c, p, d, cand, fr, im in items] + [list(collated_shape)]
+
+
+def test_variant_image_store_read_by_reference_dataloader(tmp_path):
+    f = str(tmp_path / "img.hdf5")
+    items = write_variant_images(f)
+    refdigest.expect("store_variant_images", dict(layout=layout(f), reader=variant_items(items, (2, 33, 26))))
+
+
+# ---- a16: variant prediction store -> pepper_variant CandidateFinder.small_chunk_stitch
+def write_variant_predictions(f):
+    """Writes the store; returns (genome, positions, depths, keys, freqs, probs) of its candidates."""
     rng = np.random.default_rng(2)
     L = 600
     genome = "".join("ACGT"[i] for i in rng.integers(0, 4, L))
@@ -112,53 +63,56 @@ def test_variant_prediction_store_read_by_reference_candidate_finder(tmp_path, r
         keys.append("1" + "ACGT"[rng.integers(0, 4)] if t == 1 else ("2" + genome[p] + "AC" if t == 2 else "3" + genome[p:p + 3]))
     depths = rng.integers(4, 60, n); freqs = np.minimum(depths, rng.integers(1, 30, n))
     probs = rng.dirichlet([0.6, 0.5, 0.4], n).astype(np.float32)
-
-    class FASTA_handler:
-        def __init__(self, path):
-            pass
-
-        def get_reference_sequence(self, contig, a, b):
-            return genome[max(0, a):max(0, b)]
-    ref_modules.FASTA_handler = FASTA_handler
-    from pepper_variant.modules.python import CandidateFinder as RefCF
-    f = str(tmp_path / "pred.hdf")
     with ds.VariantPredictionStore(f, backend="npz") as s:
         s.write_prediction(0, ["ctg"] * n, positions, depths, keys, freqs, probs)
-    options = dict(snp_p_value=0.1, insert_p_value=0.1, delete_p_value=0.1, snp_p_value_in_lc=0.3, insert_p_value_in_lc=0.35,
-                   delete_p_value_in_lc=0.25, report_snp_above_freq=0.0, report_indel_above_freq=0.6)
-    got_m, got_d = RefCF.small_chunk_stitch(types.SimpleNamespace(fasta="x", **options), [(f, "batch_0")])
-    want_m, want_d = ofc.select(options, "ctg", positions, depths, keys, freqs, probs.astype(np.float64), lambda c, a, b: genome[max(0, a):max(0, b)])
-    assert len(got_d) == len(want_d) > 20 and len(got_m) == len(want_m) > 5       # fixed-bytes candidates would drop every record
-    for a, b in zip(got_d, want_d):
-        assert (a[0], int(a[1]), int(a[2]), a[3], a[4], a[5], int(a[6]), [int(x) for x in a[7]], bool(a[11])) == \
-               (b[0], b[1], b[2], b[3], b[4], b[5], b[6], b[7], b[11])
-        assert abs(float(a[8]) - float(b[8])) < 1e-12
+    return genome, positions, depths, keys, freqs, probs
 
 
-def test_polish_image_store_read_by_reference_dataloader(tmp_path, ref_modules):
-    from pepper_b200 import datastore as ds
-    from pepper.modules.python.models.dataloader_predict import SequenceDataset
-    f = str(tmp_path / "pimg.hdf")
+def candidate_records(margin, deepvariant):
+    return [len(margin), [[_s(a[0]), int(a[1]), int(a[2]), _s(a[3]), _s(a[4]), _s(a[5]), int(a[6]), [int(x) for x in a[7]],
+                           round(float(a[8]), 9), bool(a[11])] for a in deepvariant]]
+
+
+def test_variant_prediction_store_read_by_reference_candidate_finder(tmp_path):
+    from oracle import find_candidates as ofc
+    f = str(tmp_path / "pred.hdf")
+    genome, positions, depths, keys, freqs, probs = write_variant_predictions(f)
+    want_m, want_d = ofc.select(VARIANT_OPTIONS, "ctg", positions, depths, keys, freqs, probs.astype(np.float64),
+                                lambda c, a, b: genome[max(0, a):max(0, b)])
+    assert len(want_d) > 20 and len(want_m) > 5               # fixed-bytes candidates would drop every record
+    refdigest.expect("store_variant_predictions", dict(layout=layout(f), reader=candidate_records(want_m, want_d)))
+
+
+# ---- a12: polish image store -> pepper dataloader_predict.SequenceDataset
+def write_polish_images(f):
+    """Writes the store; returns the (contig, chunk start, chunk end, chunk id, image, position) items it must read back as."""
     img = (np.arange(10000) % 255).astype(np.uint8).reshape(1000, 10)
     with ds.PolishImageStore(f, backend="npz") as s:
         s.write_summary("ctg1", 0, 1100, 1, img, np.arange(1000), np.zeros(1000, np.int64))
-    data = SequenceDataset(None, file_list=[f])
-    assert len(data) == 1
-    contig, cs, ce, cid, image, position, index = data[0]
-    assert isinstance(contig, str) and contig == "ctg1" and "b'" not in (contig + "-" + str(cs))
-    assert (int(cs), int(ce), int(cid)) == (0, 1100, 1) and np.array_equal(image, img) and position.dtype == np.int64
+    return [("ctg1", 0, 1100, 1, img, np.arange(1000, dtype=np.int64))]
 
 
-def test_polish_prediction_store_read_by_reference_stitch(tmp_path, ref_modules):
-    from pepper_b200 import datastore as ds
-    from oracle import stitch as ostitch
-    from pepper.modules.python import Stitch as RefStitch
+def polish_items(items):
+    return [[_s(c), int(cs), int(ce), int(cid), np.asarray(im).astype(np.int64).tolist(), np.asarray(pos).dtype.str]
+            for c, cs, ce, cid, im, pos in items]
+
+
+def test_polish_image_store_read_by_reference_dataloader(tmp_path):
+    f = str(tmp_path / "pimg.hdf")
+    items = write_polish_images(f)
+    refdigest.expect("store_polish_images", dict(layout=layout(f), reader=polish_items(items)))
+
+
+# ---- a14: polish prediction store -> pepper Stitch.small_chunk_stitch
+POLISH_REGIONS = [(0, 1100), (900, 2000)]
+
+
+def write_polish_predictions(f):
+    """Writes the store; returns its images as (region, chunk id, position, index, bases)."""
     rng = np.random.default_rng(3)
-    regions = [(0, 1100), (900, 2000)]
-    f = str(tmp_path / "ppred.hdf")
     imgs = []
     with ds.PolishPredictionStore(f, backend="npz") as s:
-        for r, (a, b) in enumerate(regions):
+        for r, (a, b) in enumerate(POLISH_REGIONS):
             n = b - a + 1
             start, end, cid = 0, min(n, 1000), 0
             while True:
@@ -170,7 +124,15 @@ def test_polish_prediction_store_read_by_reference_stitch(tmp_path, ref_modules)
                 if end == n:
                     break
                 start = end - 50; end = min(n, start + 1000)
-    first, last, seq = RefStitch.small_chunk_stitch("ctg1", [(f, "ctg1", a, b) for a, b in regions])
+    return imgs
+
+
+def test_polish_prediction_store_read_by_reference_stitch(tmp_path):
+    from oracle import stitch as ostitch
+    f = str(tmp_path / "ppred.hdf")
+    imgs = write_polish_predictions(f)
     want = ostitch.stitch(np.stack([i[4] for i in imgs]), np.stack([i[2] for i in imgs]), np.stack([i[3] for i in imgs]),
-                          np.array([i[0] for i in imgs]), np.array([i[1] for i in imgs]), [r[0] for r in regions], [r[1] for r in regions])
-    assert seq == want and len(seq) > 1000
+                          np.array([i[0] for i in imgs]), np.array([i[1] for i in imgs]), [r[0] for r in POLISH_REGIONS],
+                          [r[1] for r in POLISH_REGIONS])
+    assert len(want) > 1000
+    refdigest.expect("store_polish_predictions", dict(layout=layout(f), reader=want))

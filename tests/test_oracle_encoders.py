@@ -1,55 +1,38 @@
 """CPU tests: the plain-C restatement (oracle/port_encoders.c) against the UNMODIFIED reference C++
-compiled into oracle/_ref, on the hand-written KATs and on seeded synthetic regions; and both against
-the committed golden fixtures (tests/golden/, produced by tests/golden/make_golden.py from oracle/_ref)."""
+compiled into oracle/_ref, on the hand-written KATs and on seeded synthetic regions (through the digests of its outputs,
+tests/golden/refdigest.py); and against the committed golden fixtures (tests/golden/, produced by
+tests/golden/make_golden.py from oracle/_ref)."""
 import os
 import numpy as np
 import pytest
 
 from pepper_b200 import synth
 from tests import kats
+from tests.golden import refdigest
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
-def _same_variant(a, b):
-    assert a["keys"] == b["keys"]
-    for k in ("images", "positions", "depths", "freqs", "region_of"):
-        assert np.array_equal(a[k], b[k]), k
-
-
-def _need_ref(oracle):
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-
-
 @pytest.mark.parametrize("idx", range(12))
 def test_variant_kat_port_vs_reference(oracle_built, idx):
-    _need_ref(oracle_built)
     name, reads, regions, params = kats.variant_kats()[idx]
     a = oracle_built.variant_encode(reads, regions, params, "port")
-    b = oracle_built.variant_encode(reads, regions, params, "ref")
-    _same_variant(a, b)
+    refdigest.expect("variant_kat_%d" % idx, refdigest.variant_fields(a, oracle_built.images_to_int8))
     assert len(a["keys"]) > 0 or name in ("refskip_pad_fallthrough",), name
 
 
 @pytest.mark.parametrize("platform,params,seed", [(synth.ONT, synth.ont_params(), 3), (synth.HIFI, synth.hifi_params(), 4)])
 def test_variant_synthetic_port_vs_reference(oracle_built, platform, params, seed):
-    _need_ref(oracle_built)
     reads, regions = synth.make_variant_workload(2, 6000, 30, platform, seed=seed)
     a = oracle_built.variant_encode(reads, regions, params, "port")
-    b = oracle_built.variant_encode(reads, regions, params, "ref")
-    _same_variant(a, b)
+    refdigest.expect("variant_synthetic_seed%d" % seed, refdigest.variant_fields(a, oracle_built.images_to_int8))
     assert len(a["keys"]) > 10
 
 
 @pytest.mark.parametrize("idx", range(4))
 def test_polish_kat_port_vs_reference(oracle_built, idx):
-    _need_ref(oracle_built)
     name, reads, regions = kats.polish_kats()[idx]
-    a = oracle_built.polish_encode(reads, regions, "port")
-    b = oracle_built.polish_encode(reads, regions, "ref")
-    for k in a:
-        assert np.array_equal(a[k], b[k]), (name, k)
+    refdigest.expect("polish_kat_%d" % idx, oracle_built.polish_encode(reads, regions, "port"))
 
 
 def test_polish_wrap_quirk(oracle_built):
@@ -64,12 +47,8 @@ def test_polish_wrap_quirk(oracle_built):
 
 
 def test_polish_synthetic_port_vs_reference(oracle_built):
-    _need_ref(oracle_built)
     reads, regions = synth.make_polish_workload(4, 40, synth.ONT, seed=9)
-    a = oracle_built.polish_encode(reads, regions, "port")
-    b = oracle_built.polish_encode(reads, regions, "ref")
-    for k in a:
-        assert np.array_equal(a[k], b[k]), k
+    refdigest.expect("polish_synthetic_seed9", oracle_built.polish_encode(reads, regions, "port"))
 
 
 def test_golden_variant(oracle_built):

@@ -1,6 +1,7 @@
 """CPU tests for row a2 (BAM_handler::get_reads): the plain-C restatement (oracle/port_getreads.c) against the UNMODIFIED
-reference function compiled into oracle/_ref/libref_getreads.so, on the branch KATs and on seeded synthetic contigs; both
-against the committed golden fixture; and the reservoir sampler against the reference's literal loop."""
+reference function compiled into oracle/_ref/libref_getreads.so, on the branch KATs and on seeded synthetic contigs (through
+the digests of its outputs, tests/golden/refdigest.py); against the committed golden fixture; and the reservoir sampler
+against the reference's literal loop."""
 import os
 import numpy as np
 import pytest
@@ -8,32 +9,28 @@ import pytest
 from pepper_b200 import synth
 from pepper_b200.reads import reservoir_select, RANDOM_SEED
 from tests import kats
-from tests.golden import make_golden_getreads as gold
+from tests.golden import make_golden_getreads as gold, refdigest
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "getreads_seed31.npz")
 FIELDS = ("pos", "seq_off", "cigar_off", "flags", "mapq", "seq", "qual", "cigar")
 
 
-def same_reads(a, b, ctx=""):
-    for f in FIELDS:
-        x, y = getattr(a, f), getattr(b, f)
-        assert np.array_equal(x, y), (ctx, f, x[:8], y[:8])
-
-
-def _need_ref(oracle):
-    if not oracle.have_ref_getreads():
-        pytest.skip("oracle/_ref/libref_getreads.so not built (needs /root/reference)")
+def synthetic_queries(seed):
+    """25 seeded get_reads queries over the synthetic contig of test_getreads_synthetic_port_vs_reference."""
+    start = 7000
+    rng = np.random.default_rng(seed)
+    for _ in range(25):
+        s = int(rng.integers(start - 500, start + 20500))
+        e = s + int(rng.choice([1, 2, 50, 1201, 6000]))
+        yield s, e, bool(rng.integers(0, 2)), int(rng.choice([0, 0, 10])), int(rng.choice([0, 7]))
 
 
 def test_getreads_kats_port_vs_reference(oracle_built):
-    _need_ref(oracle_built)
     for name, rec, queries in kats.getreads_kats():
         kept_any = 0
-        for q in queries:
+        for qi, q in enumerate(queries):
             a, ae, ab = oracle_built.get_reads(rec, *q, impl="port")
-            b, be, bb = oracle_built.get_reads(rec, *q, impl="ref")
-            same_reads(a, b, (name, q))
-            assert np.array_equal(ae, be) and np.array_equal(ab, bb), (name, q)
+            refdigest.expect("getreads_kat_%s_%d" % (name, qi), refdigest.reads_fields(a, ae, ab))
             kept_any += a.n_reads
         assert kept_any > 20
 
@@ -66,19 +63,11 @@ def test_getreads_kat_expectations(oracle_built):
 
 @pytest.mark.parametrize("seed,platform", [(3, synth.ONT), (4, synth.HIFI)])
 def test_getreads_synthetic_port_vs_reference(oracle_built, seed, platform):
-    _need_ref(oracle_built)
-    start = 7000
-    rec, _ = synth.simulate_contig_records(20000, 15, platform, seed, contig_start=start)
-    rng = np.random.default_rng(seed)
+    rec, _ = synth.simulate_contig_records(20000, 15, platform, seed, contig_start=7000)
     total = 0
-    for _ in range(25):
-        s = int(rng.integers(start - 500, start + 20500))
-        e = s + int(rng.choice([1, 2, 50, 1201, 6000]))
-        supp, mq, bq = bool(rng.integers(0, 2)), int(rng.choice([0, 0, 10])), int(rng.choice([0, 7]))
-        a, ae, ab = oracle_built.get_reads(rec, s, e, supp, mq, bq, impl="port")
-        b, be, bb = oracle_built.get_reads(rec, s, e, supp, mq, bq, impl="ref")
-        same_reads(a, b, (s, e))
-        assert np.array_equal(ae, be) and np.array_equal(ab, bb)
+    for qi, q in enumerate(synthetic_queries(seed)):
+        a, ae, ab = oracle_built.get_reads(rec, *q, impl="port")
+        refdigest.expect("getreads_synthetic_seed%d_%d" % (seed, qi), refdigest.reads_fields(a, ae, ab))
         total += a.n_reads
     assert total > 50
 

@@ -5,6 +5,7 @@ import pytest
 
 from pepper_b200 import synth
 from tests import kats
+from tests.golden import refdigest
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -18,8 +19,8 @@ def enc():
     e.close()
 
 
-def _compare(oracle, enc, reads, regions, name="", impl="port"):
-    want = oracle.polish_encode(reads, regions, impl)
+def _compare(oracle, enc, reads, regions, name=""):
+    want = oracle.polish_encode(reads, regions, "port")
     got = enc.encode(reads, regions)
     assert np.array_equal(got.col_off, want["col_off"]), name
     assert np.array_equal(got.pos, want["pos"]), name
@@ -42,11 +43,11 @@ def test_synthetic(oracle_built, enc, platform, seed, nreg, cov):
     assert got.image.shape[0] > 1000 * nreg
 
 
-def test_against_compiled_reference(oracle_built, enc):
-    if not oracle_built.have_ref():
-        pytest.skip("oracle/_ref not present")
+def test_against_compiled_reference(enc):
+    """Against the digests of the reference encoder's outputs (tests/golden/refdigest.py) on the same workload."""
     reads, regions = synth.make_polish_workload(5, 40, synth.ONT, seed=13)
-    _compare(oracle_built, enc, reads, regions, "ref", impl="ref")
+    got = enc.encode(reads, regions)
+    refdigest.expect("gpu_polish_encoder_seed13", dict(image=got.image, pos=got.pos, idx=got.idx, col_off=got.col_off))
 
 
 def test_golden(enc):

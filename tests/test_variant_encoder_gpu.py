@@ -5,6 +5,7 @@ import pytest
 
 from pepper_b200 import synth
 from tests import kats
+from tests.golden import refdigest
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -18,21 +19,20 @@ def enc():
     e.close()
 
 
-def _compare(oracle, enc, reads, regions, params, name="", impl="port"):
-    want = oracle.variant_encode(reads, regions, params, impl, debug=(impl == "port"))
+def _compare(oracle, enc, reads, regions, params, name=""):
+    want = oracle.variant_encode(reads, regions, params, "port", debug=True)
     got = enc.encode(reads, regions, params)
     # intermediates first: they localise a mismatch
-    if impl == "port":
-        for r in range(regions.n_regions):
-            L1 = int(regions.table[r, 1] - regions.table[r, 0] + 1)
-            m, cov, snp, ins, dele = enc.debug_region(r, L1)
-            wm, wcov, wsnp, wins, wdel = want["debug"][r]
-            assert np.array_equal(cov, wcov), (name, "coverage", np.nonzero(cov != wcov)[0][:10])
-            assert np.array_equal(snp, wsnp), (name, "snp_count", np.nonzero(snp != wsnp)[0][:10])
-            assert np.array_equal(ins, wins), (name, "insert_count", np.nonzero(ins != wins)[0][:10])
-            assert np.array_equal(dele, wdel), (name, "delete_count", np.nonzero(dele != wdel)[0][:10])
-            bad = np.argwhere(m != wm)
-            assert bad.size == 0, (name, "matrix", bad[:10], m[bad[0][0]], wm[bad[0][0]])
+    for r in range(regions.n_regions):
+        L1 = int(regions.table[r, 1] - regions.table[r, 0] + 1)
+        m, cov, snp, ins, dele = enc.debug_region(r, L1)
+        wm, wcov, wsnp, wins, wdel = want["debug"][r]
+        assert np.array_equal(cov, wcov), (name, "coverage", np.nonzero(cov != wcov)[0][:10])
+        assert np.array_equal(snp, wsnp), (name, "snp_count", np.nonzero(snp != wsnp)[0][:10])
+        assert np.array_equal(ins, wins), (name, "insert_count", np.nonzero(ins != wins)[0][:10])
+        assert np.array_equal(dele, wdel), (name, "delete_count", np.nonzero(dele != wdel)[0][:10])
+        bad = np.argwhere(m != wm)
+        assert bad.size == 0, (name, "matrix", bad[:10], m[bad[0][0]], wm[bad[0][0]])
     assert got.keys == want["keys"], (name, got.keys[:10], want["keys"][:10])
     assert np.array_equal(got.positions, want["positions"]), name
     assert np.array_equal(got.depths.astype(np.int32), want["depths"]), name
@@ -63,11 +63,13 @@ def test_synthetic(oracle_built, enc, platform, params, seed, nreg, size):
     assert len(got) > 10
 
 
-def test_against_compiled_reference(oracle_built, enc):
-    if not oracle_built.have_ref():
-        pytest.skip("oracle/_ref not present")
+def test_against_compiled_reference(enc):
+    """Against the digests of the reference encoder's outputs (tests/golden/refdigest.py) on the same workload."""
     reads, regions = synth.make_variant_workload(2, 8000, 30, synth.ONT, seed=8)
-    _compare(oracle_built, enc, reads, regions, synth.ont_params(), "ref", impl="ref")
+    got = enc.encode(reads, regions, synth.ont_params())
+    refdigest.expect("gpu_variant_encoder_seed8", dict(keys=got.keys, positions=got.positions, depths=got.depths, freqs=got.freqs,
+                                                       region_of=got.region_of, images_i8=got.images))
+    assert np.array_equal(got.n_per_region, np.bincount(got.region_of.astype(np.int64), minlength=regions.n_regions))
 
 
 def test_ref_with_N_blocks(oracle_built, enc):
