@@ -407,11 +407,17 @@ int pb_polish_net_launches(pb_polish_net_t *net, int64_t *n_launches);
  * everywhere; DESIGN.md section 4 holds the measured error of every choice.                                                     */
 int pb_variant_net_set_lo_mask(pb_variant_net_t *net, int mask);
 int pb_polish_net_set_lo_mask(pb_polish_net_t *net, int mask);
+/* Variant network, same bits as lo_mask: a set bit runs that GEMM's correction products (a_hi*w_lo, and a_lo*w_hi where lo_mask
+ * keeps it) as e4m3 tensor-core MMAs (kind::f8f6f4) next to the fp16 main product; default 0x1f.  0 = the fp16 split everywhere. */
+int pb_variant_net_set_f8_mask(pb_variant_net_t *net, int mask);
 /* 0 = fp32 FFMA GEMMs, 1 = tcgen05 GEMMs with the fp16 hi/lo operand split x3 (fp32-equivalent, default) */
 int pb_polish_net_set_mode(pb_polish_net_t *net, int mode);
 
 /* diagnostics: C[M][N] = A[M][K] W[N][K]^T + bias through the tcgen05 kernel (N % 256 == 0, K % 32 == 0) */
 int pb_test_tc_gemm(int M, int N, int K, const float *h_A, const float *h_W, const float *h_bias, float *h_out);
+/* the same GEMM with the variant network's operand images: weights scaled by 2^(12-E) (max|w| = f * 2^E, f in [0.5, 1)) with
+ * e4m3 copies; lo = 1 runs a_lo*w_hi, f8 = 1 runs the corrections in e4m3 */
+int pb_test_tc_gemm_f8(int M, int N, int K, const float *h_A, const float *h_W, const float *h_bias, float *h_out, int lo, int f8);
 
 /* ------------------------------------------------------------------------
  * Fused make_images + run_inference for the variant path: what

@@ -8,18 +8,24 @@ struct VariantStream;      // streaming session state (pipeline.cu)
 struct DevRnn { DevBuf W, bias; int K0, K0p, K1, Kp, H; };
 struct DevLin { DevBuf W, bias; int N, K, Kp; };
 // tcgen05 path (nets_tc.cu): weights as bf16 hi/lo tile images + per-chunk tiled operands
-struct TcRnn { DevBuf w_hi, w_lo; int nkt_x = 0, nkt_h = 0; };
-struct TcLin { DevBuf w_hi, w_lo; int nkt = 0; };
+// with_f8 uploads (variant) also hold e4m3 images, and their fp16 images are scaled: accumulator x acc_scale = GEMM value
+// (tc_gemm.cuh, "e4m3 correction operands")
+struct TcRnn { DevBuf w_hi, w_lo, w8_hi, w8_lo; float acc_scale = 1.f; int nkt_x = 0, nkt_h = 0; };
+struct TcLin { DevBuf w_hi, w_lo, w8_hi, w8_lo; float acc_scale = 1.f; int nkt = 0; };
 struct TcVariant {
     TcRnn enc[2], dec[2];
     TcLin lin[5];
     DevBuf img_op, yenc_hi, yenc_lo, ydec_hi, ydec_lo, c, act_hi[2], act_lo[2], final_f32;
+    DevBuf img_op8, yenc_hi8, yenc_lo8, ydec_hi8, ydec_lo8, act_hi8[2], act_lo8[2];      // e4m3 images of the same operands
     // which GEMMs execute the third (a_lo x w_hi) product: bit 0 encoder h-part, 1 decoder x-part, 2 decoder h-part, 3 linear_1,
     // 4 linear_2..5; clearing a bit runs that GEMM with two products, 0x1f = three everywhere.  Default 0x1a: the recurrent
     // (h-part) GEMMs of both LSTM layers run with two products — each passes the parity gate on its own (hidden states within
     // 1e-3, class index exact outside the 1e-4 margin; DESIGN.md section 4 has the per-GEMM errors) — while the decoder's x-part
     // and the MLP head, which fail it, keep three.
     int lo_mask = 0x1a;
+    // same bit order: a set bit runs that GEMM's correction products (a_hi x w_lo, and a_lo x w_hi where lo_mask keeps it) as
+    // e4m3 MMAs instead of fp16 ones.  0 = the fp16 split everywhere (the cross-check).
+    int f8_mask = 0x1f;
 };
 struct TcPolish {
     TcRnn enc[2], dec[2];
@@ -39,8 +45,8 @@ struct OutSink {
         return S;
     }
 };
-int tc_upload_rnn(TcRnn &T, const float *Wp, int K0, int K0p_src, int H, int Kp_src);
-int tc_upload_lin(TcLin &T, const float *w, int N, int K);
+int tc_upload_rnn(TcRnn &T, const float *Wp, int K0, int K0p_src, int H, int Kp_src, bool with_f8);
+int tc_upload_lin(TcLin &T, const float *w, int N, int K, bool with_f8);
 }  // namespace pb
 
 struct pb_variant_encoder {

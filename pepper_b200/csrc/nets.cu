@@ -391,14 +391,14 @@ extern "C" int pb_variant_net_create(pb_variant_net_t **out, int device, const f
         const PackedRnn pd = pack_lstm(P[8 + 4 * d + 0], P[8 + 4 * d + 1], P[8 + 4 * d + 2], P[8 + 4 * d + 3], 512, VH);
         PB_TRY(upload_rnn(N->enc[d], pe));
         PB_TRY(upload_rnn(N->dec[d], pd));
-        PB_TRY(tc_upload_rnn(N->tc->enc[d], pe.W.data(), pe.K0, pe.K0p, VH, pe.Kp));
-        PB_TRY(tc_upload_rnn(N->tc->dec[d], pd.W.data(), pd.K0, pd.K0p, VH, pd.Kp));
+        PB_TRY(tc_upload_rnn(N->tc->enc[d], pe.W.data(), pe.K0, pe.K0p, VH, pe.Kp, true));
+        PB_TRY(tc_upload_rnn(N->tc->dec[d], pd.W.data(), pd.K0, pd.K0p, VH, pd.Kp, true));
     }
     PB_TRY(upload_lin(N->lin[0], P[16], P[17], 512, VT * 512));
-    PB_TRY(tc_upload_lin(N->tc->lin[0], P[16], 512, VT * 512));
+    PB_TRY(tc_upload_lin(N->tc->lin[0], P[16], 512, VT * 512, true));
     for (int i = 1; i < 5; i++) {
         PB_TRY(upload_lin(N->lin[i], P[16 + 2 * i], P[17 + 2 * i], 512, 512));
-        PB_TRY(tc_upload_lin(N->tc->lin[i], P[16 + 2 * i], 512, 512));
+        PB_TRY(tc_upload_lin(N->tc->lin[i], P[16 + 2 * i], 512, 512, true));
     }
     PB_TRY(upload_lin(N->outl, P[26], P[27], 3, 512));
     *out = N;
@@ -414,9 +414,11 @@ extern "C" int pb_variant_net_destroy(pb_variant_net_t *N) {
     for (auto *b : bufs) b->release();
     if (N->tc) {
         TcVariant &T = *N->tc;
-        for (int d = 0; d < 2; d++) { T.enc[d].w_hi.release(); T.enc[d].w_lo.release(); T.dec[d].w_hi.release(); T.dec[d].w_lo.release(); }
-        for (auto &l : T.lin) { l.w_hi.release(); l.w_lo.release(); }
-        DevBuf *tb[] = {&T.img_op, &T.yenc_hi, &T.yenc_lo, &T.ydec_hi, &T.ydec_lo, &T.c, &T.act_hi[0], &T.act_hi[1], &T.act_lo[0], &T.act_lo[1], &T.final_f32};
+        for (int d = 0; d < 2; d++)
+            for (TcRnn *r : {&T.enc[d], &T.dec[d]}) { r->w_hi.release(); r->w_lo.release(); r->w8_hi.release(); r->w8_lo.release(); }
+        for (auto &l : T.lin) { l.w_hi.release(); l.w_lo.release(); l.w8_hi.release(); l.w8_lo.release(); }
+        DevBuf *tb[] = {&T.img_op, &T.yenc_hi, &T.yenc_lo, &T.ydec_hi, &T.ydec_lo, &T.c, &T.act_hi[0], &T.act_hi[1], &T.act_lo[0], &T.act_lo[1], &T.final_f32,
+                        &T.img_op8, &T.yenc_hi8, &T.yenc_lo8, &T.ydec_hi8, &T.ydec_lo8, &T.act_hi8[0], &T.act_hi8[1], &T.act_lo8[0], &T.act_lo8[1]};
         for (auto *b : tb) b->release();
         delete N->tc;
     }
@@ -434,6 +436,12 @@ extern "C" int pb_variant_net_set_mode(pb_variant_net_t *N, int mode) {
 extern "C" int pb_variant_net_set_lo_mask(pb_variant_net_t *N, int mask) {
     if (!N || !N->tc) { set_error("no tcgen05 state"); return PB_ERR_ARG; }
     N->tc->lo_mask = mask & 0x1f;
+    return PB_OK;
+}
+// which GEMMs run their correction products as e4m3 MMAs (same bits; 0 = the fp16 split everywhere)
+extern "C" int pb_variant_net_set_f8_mask(pb_variant_net_t *N, int mask) {
+    if (!N || !N->tc) { set_error("no tcgen05 state"); return PB_ERR_ARG; }
+    N->tc->f8_mask = mask & 0x1f;
     return PB_OK;
 }
 extern "C" int pb_polish_net_set_lo_mask(pb_polish_net_t *N, int mask) {
@@ -609,8 +617,8 @@ extern "C" int pb_polish_net_create(pb_polish_net_t **out, int device, const flo
         const PackedRnn pd = pack_gru(P[8 + 4 * d + 0], P[8 + 4 * d + 1], P[8 + 4 * d + 2], P[8 + 4 * d + 3], 256, PH);
         PB_TRY(upload_rnn(N->enc[d], pe));
         PB_TRY(upload_rnn(N->dec[d], pd));
-        PB_TRY(tc_upload_rnn(N->tc->enc[d], pe.W.data(), pe.K0, pe.K0p, PH, pe.Kp));
-        PB_TRY(tc_upload_rnn(N->tc->dec[d], pd.W.data(), pd.K0, pd.K0p, PH, pd.Kp));
+        PB_TRY(tc_upload_rnn(N->tc->enc[d], pe.W.data(), pe.K0, pe.K0p, PH, pe.Kp, false));
+        PB_TRY(tc_upload_rnn(N->tc->dec[d], pd.W.data(), pd.K0, pd.K0p, PH, pd.Kp, false));
     }
     PB_TRY(N->dW.reserve(sizeof(float) * 5 * 256));
     PB_TRY(N->dB.reserve(sizeof(float) * 8));

@@ -18,20 +18,37 @@ namespace pb {
 static inline uint16_t f2bf(float f) { return tc::op_bits(f); }      // round to nearest even into the operand type
 static inline float bf2f(uint16_t h) { return tc::op_val(h); }
 
-// row-major [rows][K] fp32 (rows % 128 == 0 after padding, K % 32 == 0 after padding) -> hi / lo tiles [rt][kt][4][128][8]
+// row-major [rows][K] fp32 (rows % 128 == 0 after padding, K % 32 == 0 after padding) -> hi / lo tiles [rt][kt][4][128][8] of
+// v = src * scale.  With F8 set, also the e4m3 tiles [rt][kt][2][128][16]: hi8 = e4m3(v * F8->hi_scale), lo8 = e4m3((v - v_hi) *
+// F8->lo_scale) — (2^-12, 1) for weights, (1, 2^12) for activations (tc_gemm.cuh, "e4m3 correction operands").
+struct F8Tiles {
+    std::vector<uint8_t> hi, lo;
+    float hi_scale, lo_scale;
+};
 static void tile_matrix(const float *src, int64_t rows, int64_t K, int64_t rows_p, int64_t Kp, std::vector<uint16_t> &hi, std::vector<uint16_t> &lo,
-                        int64_t TR = 128 /* rows per tile: 128 for A operands, 256 for the weights of the persistent kernel */) {
+                        int64_t TR = 128 /* rows per tile: 128 for A operands, 256 for the weights of the persistent kernel */,
+                        float scale = 1.f, F8Tiles *F8 = nullptr) {
     const int64_t RT = rows_p / TR, KT = Kp / 32;
     hi.assign((size_t) (RT * KT * TR * 32), 0);
     lo.assign((size_t) (RT * KT * TR * 32), 0);
+    if (F8) {
+        F8->hi.assign(hi.size(), 0);
+        F8->lo.assign(hi.size(), 0);
+    }
     for (int64_t r = 0; r < rows; r++)
         for (int64_t k = 0; k < K; k++) {
-            const float v = src[r * K + k];
+            const float v = src[r * K + k] * scale;
             const uint16_t h = f2bf(v);
-            const uint16_t l = f2bf(v - bf2f(h));
-            const int64_t o = ((r / TR) * KT + k / 32) * (TR * 32) + ((k % 32) / 8) * (TR * 8) + (r % TR) * 8 + (k % 8);
+            const float res = v - bf2f(h);
+            const int64_t tile = ((r / TR) * KT + k / 32) * (TR * 32);
+            const int64_t o = tile + ((k % 32) / 8) * (TR * 8) + (r % TR) * 8 + (k % 8);
             hi[(size_t) o] = h;
-            lo[(size_t) o] = l;
+            lo[(size_t) o] = f2bf(res);
+            if (F8) {
+                const int64_t o8 = tile + ((k % 32) / 16) * (TR * 16) + (r % TR) * 16 + (k % 16);
+                F8->hi[(size_t) o8] = tc::f8_bits(v * F8->hi_scale);
+                F8->lo[(size_t) o8] = tc::f8_bits(res * F8->lo_scale);
+            }
         }
 }
 
@@ -42,9 +59,37 @@ static int upload_tiles(DevBuf &dhi, DevBuf &dlo, const std::vector<uint16_t> &h
     PB_CUDA(cudaMemcpy(dlo.p, lo.data(), lo.size() * 2, cudaMemcpyHostToDevice));
     return PB_OK;
 }
+static int upload_f8(DevBuf &dhi, DevBuf &dlo, const F8Tiles &F) {
+    PB_TRY(dhi.reserve(F.hi.size()));
+    PB_TRY(dlo.reserve(F.lo.size()));
+    PB_CUDA(cudaMemcpy(dhi.p, F.hi.data(), F.hi.size(), cudaMemcpyHostToDevice));
+    PB_CUDA(cudaMemcpy(dlo.p, F.lo.data(), F.lo.size(), cudaMemcpyHostToDevice));
+    return PB_OK;
+}
+
+// Weight images, optionally with the e4m3 correction images: the fp16 images then hold w * 2^(12-E), max|w * 2^-E| in
+// [0.5, 1), and *acc_scale = 2^(E-12) maps the accumulator back.
+static int upload_weight(const float *w, int64_t N, int64_t K, int64_t Np, int64_t Kp, bool with_f8, DevBuf &w_hi, DevBuf &w_lo, DevBuf &w8_hi,
+                         DevBuf &w8_lo, float &acc_scale) {
+    std::vector<uint16_t> hi, lo;
+    if (!with_f8) {
+        tile_matrix(w, N, K, Np, Kp, hi, lo, 256);
+        acc_scale = 1.f;
+        return upload_tiles(w_hi, w_lo, hi, lo);
+    }
+    float m = 0.f;
+    for (int64_t i = 0; i < N * K; i++) m = std::max(m, fabsf(w[i]));
+    int E = 0;
+    if (m > 0.f) frexpf(m, &E);                              // m = f * 2^E, f in [0.5, 1)
+    F8Tiles F{{}, {}, 1.f / tc::F8_LO_SCALE, 1.f};
+    tile_matrix(w, N, K, Np, Kp, hi, lo, 256, ldexpf(1.f, 12 - E), &F);
+    acc_scale = ldexpf(1.f, E - 12);
+    PB_TRY(upload_tiles(w_hi, w_lo, hi, lo));
+    return upload_f8(w8_hi, w8_lo, F);
+}
 
 // weights of one RNN direction, packed rows 4j+g (host copy kept by nets.cu) with K = [x | pad32 | h]
-int tc_upload_rnn(TcRnn &T, const float *Wp /* [4H][Kp_src] */, int K0, int K0p_src, int H, int Kp_src) {
+int tc_upload_rnn(TcRnn &T, const float *Wp /* [4H][Kp_src] */, int K0, int K0p_src, int H, int Kp_src, bool with_f8) {
     const int K0p = (K0 + 31) / 32 * 32;
     const int Kp = K0p + H;
     std::vector<float> W((size_t) 4 * H * Kp, 0.f);
@@ -52,17 +97,13 @@ int tc_upload_rnn(TcRnn &T, const float *Wp /* [4H][Kp_src] */, int K0, int K0p_
         for (int k = 0; k < K0; k++) W[(size_t) n * Kp + k] = Wp[(size_t) n * Kp_src + k];
         for (int k = 0; k < H; k++) W[(size_t) n * Kp + K0p + k] = Wp[(size_t) n * Kp_src + K0p_src + k];
     }
-    std::vector<uint16_t> hi, lo;
-    tile_matrix(W.data(), 4 * H, Kp, 4 * H, Kp, hi, lo, 256);
     T.nkt_x = K0p / 32; T.nkt_h = H / 32;
-    return upload_tiles(T.w_hi, T.w_lo, hi, lo);
+    return upload_weight(W.data(), 4 * H, Kp, 4 * H, Kp, with_f8, T.w_hi, T.w_lo, T.w8_hi, T.w8_lo, T.acc_scale);
 }
-int tc_upload_lin(TcLin &T, const float *w, int N, int K) {
-    std::vector<uint16_t> hi, lo;
+int tc_upload_lin(TcLin &T, const float *w, int N, int K, bool with_f8) {
     const int Np = (N + 255) / 256 * 256, Kp = (K + 31) / 32 * 32;
-    tile_matrix(w, N, K, Np, Kp, hi, lo, 256);
     T.nkt = Kp / 32;
-    return upload_tiles(T.w_hi, T.w_lo, hi, lo);
+    return upload_weight(w, N, K, Np, Kp, with_f8, T.w_hi, T.w_lo, T.w8_hi, T.w8_lo, T.acc_scale);
 }
 
 static int g_num_sms = 0;
@@ -89,11 +130,28 @@ static int launch_tc(const Args &A, int mt, int nt128, int ndir, cudaStream_t st
 static Dir empty_dir() {
     Dir D;
     memset(&D, 0, sizeof(D));
+    D.acc_scale = 1.f;
     return D;
 }
 
 // ------------------------------------------------------------------------------------------------- variant
 constexpr int VT = 33, VH = 256;
+
+// GEMM slots of lo_mask / f8_mask: 0 encoder (x- and h-part), 1 decoder x-part, 2 decoder h-part, 3 linear_1, 4 linear_2-5.
+// An operand is written in the images its consumer GEMMs (slot bits `consumers`) read: fp16 hi always, fp16 lo where an fp16
+// GEMM runs a_lo*w_hi, e4m3 hi where a GEMM runs its corrections in e4m3, e4m3 lo where such a GEMM also runs a_lo*w_hi.
+struct OpImages { bool lo16, hi8, lo8; };
+static OpImages op_images(const TcVariant &T, int consumers) {
+    OpImages r{false, false, false};
+    for (int i = 0; i < 5; i++) {
+        if (!((consumers >> i) & 1)) continue;
+        const bool lo = (T.lo_mask >> i) & 1, f8 = (T.f8_mask >> i) & 1;
+        r.lo16 |= lo && !f8;
+        r.hi8 |= f8;
+        r.lo8 |= lo && f8;
+    }
+    return r;
+}
 
 int variant_forward_tc(pb_variant_net *N, const int8_t *d_images, int64_t B, float *d_probs, float *d_hidden_dbg, cudaStream_t st,
                        void (*out_kernel)(const float *, const float *, const float *, float *, int64_t, const OutSink &, cudaStream_t),
@@ -101,44 +159,76 @@ int variant_forward_tc(pb_variant_net *N, const int8_t *d_images, int64_t B, flo
     TcVariant &T = *N->tc;
     const int64_t Mt = ceil_div(B, 128), Bp = Mt * 128;
     const int64_t seq_tiles = Mt * VT * 16;                 // [mt][t][16 k-tiles] of a 512-feature sequence operand
+    const size_t seq_bytes = (size_t) (seq_tiles * TILE_ELEMS) * 2, act_bytes = (size_t) (Mt * 16 * TILE_ELEMS) * 2;
+    const OpImages enc_out = op_images(T, 0x3), dec_out = op_images(T, 0xc), act_out = op_images(T, 0x10);
     PB_TRY(T.img_op.reserve((size_t) (Mt * VT * TILE_ELEMS) * 2));
-    PB_TRY(T.yenc_hi.reserve((size_t) (seq_tiles * TILE_ELEMS) * 2));
-    PB_TRY(T.yenc_lo.reserve((size_t) (seq_tiles * TILE_ELEMS) * 2));
-    PB_TRY(T.ydec_hi.reserve((size_t) (seq_tiles * TILE_ELEMS) * 2));
-    PB_TRY(T.ydec_lo.reserve((size_t) (seq_tiles * TILE_ELEMS) * 2));
+    PB_TRY(T.img_op8.reserve((size_t) (Mt * VT * TILE_ELEMS)));
+    PB_TRY(T.yenc_hi.reserve(seq_bytes));
+    PB_TRY(T.ydec_hi.reserve(seq_bytes));
+    if (enc_out.lo16) PB_TRY(T.yenc_lo.reserve(seq_bytes));
+    if (dec_out.lo16) PB_TRY(T.ydec_lo.reserve(seq_bytes));
+    if (enc_out.hi8) PB_TRY(T.yenc_hi8.reserve(seq_bytes / 2));
+    if (enc_out.lo8) PB_TRY(T.yenc_lo8.reserve(seq_bytes / 2));
+    if (dec_out.hi8) PB_TRY(T.ydec_hi8.reserve(seq_bytes / 2));
+    if (dec_out.lo8) PB_TRY(T.ydec_lo8.reserve(seq_bytes / 2));
     PB_TRY(T.c.reserve(sizeof(float) * 2 * VH * Bp));
     for (int i = 0; i < 2; i++) {
-        PB_TRY(T.act_hi[i].reserve((size_t) (Mt * 16 * TILE_ELEMS) * 2));
-        PB_TRY(T.act_lo[i].reserve((size_t) (Mt * 16 * TILE_ELEMS) * 2));
+        PB_TRY(T.act_hi[i].reserve(act_bytes));
+        if (act_out.lo16) PB_TRY(T.act_lo[i].reserve(act_bytes));
+        if (act_out.hi8) PB_TRY(T.act_hi8[i].reserve(act_bytes / 2));
+        if (act_out.lo8) PB_TRY(T.act_lo8[i].reserve(act_bytes / 2));
     }
     PB_TRY(T.final_f32.reserve(sizeof(float) * Bp * 512));
+    auto pick16 = [](bool want, DevBuf &b) { return want ? b.as<bf16>() : nullptr; };
+    auto pick8 = [](bool want, DevBuf &b) { return want ? b.as<uint8_t>() : nullptr; };
+    const bool img8 = (T.f8_mask & 1) != 0;                 // the encoder's x-part reads e4m3 images
 
-    tc::k_tc_pack_images<<<(unsigned) ceil_div(Bp * VT * 4, 256), 256, 0, st>>>(d_images, T.img_op.as<bf16>(), B, VT, 26);
+    tc::k_tc_pack_images<<<(unsigned) ceil_div(Bp * VT * 4, 256), 256, 0, st>>>(d_images, T.img_op.as<bf16>(), pick8(img8, T.img_op8), B, VT, 26);
     N->launches++;
 
+    // A-operand segment at tile offset `off` of a sequence / activation operand, for a GEMM with the given lo / f8 bits
+    auto seg = [](const bf16 *hi, const bf16 *lo16, const uint8_t *hi8, const uint8_t *lo8, int64_t off, int lo, int f8) {
+        Seg S;
+        memset(&S, 0, sizeof(S));
+        S.hi = hi + off;
+        if (f8) { S.hi8 = hi8 + off; S.lo8 = lo ? lo8 + off : nullptr; }
+        else S.lo = lo ? lo16 + off : nullptr;
+        return S;
+    };
     for (int layer = 0; layer < 2; layer++) {
         PB_CUDA(cudaMemsetAsync(T.c.p, 0, sizeof(float) * 2 * VH * Bp, st));
+        const OpImages &yo = layer == 0 ? enc_out : dec_out;
         bf16 *y_hi = layer == 0 ? T.yenc_hi.as<bf16>() : T.ydec_hi.as<bf16>();
-        bf16 *y_lo = layer == 0 ? T.yenc_lo.as<bf16>() : T.ydec_lo.as<bf16>();
+        bf16 *y_lo = pick16(yo.lo16, layer == 0 ? T.yenc_lo : T.ydec_lo);
+        uint8_t *y_hi8 = pick8(yo.hi8, layer == 0 ? T.yenc_hi8 : T.ydec_hi8), *y_lo8 = pick8(yo.lo8, layer == 0 ? T.yenc_lo8 : T.ydec_lo8);
+        // slot bits of this layer's x-part and h-part
+        const int sx = layer == 0 ? 0 : 1, sh = layer == 0 ? 0 : 2;
+        const int lo_x = layer == 0 ? 0 : (T.lo_mask >> sx) & 1;        // encoder x-part: int8 images are exact (no lo operand at all)
+        const int lo_h = (T.lo_mask >> sh) & 1, f8_x = (T.f8_mask >> sx) & 1, f8_h = (T.f8_mask >> sh) & 1;
         static const bool persist = !(getenv("PB_LSTM_PERSIST") && atoi(getenv("PB_LSTM_PERSIST")) == 0);
         if (persist) {
             // one launch per layer: every CTA keeps its (direction, row tile) for all 33 steps (k_lstm_layer)
             tc::LstmLayer L;
             memset(&L, 0, sizeof(L));
-            if (layer == 0) { L.x_hi = T.img_op.as<bf16>(); L.x_lo = nullptr; L.x_mt_stride = (int64_t) VT * TILE_ELEMS; L.x_nkt = 1; }
-            else { L.x_hi = T.yenc_hi.as<bf16>(); L.x_lo = T.yenc_lo.as<bf16>(); L.x_mt_stride = (int64_t) VT * 16 * TILE_ELEMS; L.x_nkt = 16; }
+            if (layer == 0) {
+                L.x_hi = T.img_op.as<bf16>(); L.x_hi8 = T.img_op8.as<uint8_t>();
+                L.x_mt_stride = (int64_t) VT * TILE_ELEMS; L.x_nkt = 1;
+            } else {
+                L.x_hi = T.yenc_hi.as<bf16>(); L.x_lo = T.yenc_lo.as<bf16>(); L.x_hi8 = T.yenc_hi8.as<uint8_t>(); L.x_lo8 = T.yenc_lo8.as<uint8_t>();
+                L.x_mt_stride = (int64_t) VT * 16 * TILE_ELEMS; L.x_nkt = 16;
+            }
             for (int d = 0; d < 2; d++) {
                 TcRnn &W = layer == 0 ? T.enc[d] : T.dec[d];
                 L.w_hi[d] = W.w_hi.as<bf16>(); L.w_lo[d] = W.w_lo.as<bf16>();
+                L.w8_hi[d] = W.w8_hi.as<uint8_t>(); L.w8_lo[d] = W.w8_lo.as<uint8_t>(); L.acc_scale[d] = W.acc_scale;
                 L.bias[d] = (layer == 0 ? N->enc[d] : N->dec[d]).bias.as<float>();
                 L.c[d] = T.c.as<float>() + (int64_t) d * VH * Bp;
                 if (W.nkt_x != L.x_nkt || W.nkt_h != 8) { set_error("unexpected packed LSTM weight shape"); return PB_ERR_STATE; }
             }
-            L.y_hi = y_hi; L.y_lo = y_lo; L.y_mt_stride = (int64_t) VT * 16 * TILE_ELEMS;
+            L.y_hi = y_hi; L.y_lo = y_lo; L.y_hi8 = y_hi8; L.y_lo8 = y_lo8; L.y_mt_stride = (int64_t) VT * 16 * TILE_ELEMS;
             if (layer == 1 && d_hidden_dbg) { L.y_f32 = d_hidden_dbg; L.ldy = (int64_t) VT * 512; }
             L.M = (int) B; L.n_mt = (int) Mt; L.T = VT; L.c_ld = Bp;
-            L.lo_x = layer == 0 ? 1 : ((T.lo_mask >> 1) & 1);       // encoder x-part: int8 images are exact (no lo operand at all)
-            L.lo_h = layer == 0 ? (T.lo_mask & 1) : ((T.lo_mask >> 2) & 1);
+            L.lo_x = lo_x; L.lo_h = lo_h; L.f8_x = f8_x; L.f8_h = f8_h;
             static bool attr_set = false;
             if (!attr_set) {
                 PB_CUDA(cudaFuncSetAttribute(tc::k_lstm_layer, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::PSMEM_BYTES));
@@ -157,20 +247,23 @@ int variant_forward_tc(pb_variant_net *N, const int8_t *d_images, int64_t B, flo
                 Dir D = empty_dir();
                 TcRnn &W = layer == 0 ? T.enc[d] : T.dec[d];
                 if (layer == 0) {
-                    D.seg[0].hi = T.img_op.as<bf16>() + (int64_t) tt * TILE_ELEMS; D.seg[0].lo = nullptr;
+                    D.seg[0] = seg(T.img_op.as<bf16>(), nullptr, T.img_op8.as<uint8_t>(), nullptr, (int64_t) tt * TILE_ELEMS, 0, f8_x);
                     D.seg[0].mt_stride = (int64_t) VT * TILE_ELEMS; D.seg[0].nkt = 1;
                 } else {
-                    D.seg[0].hi = T.yenc_hi.as<bf16>() + (int64_t) tt * 16 * TILE_ELEMS; D.seg[0].lo = T.yenc_lo.as<bf16>() + (int64_t) tt * 16 * TILE_ELEMS;
+                    D.seg[0] = seg(T.yenc_hi.as<bf16>(), T.yenc_lo.as<bf16>(), T.yenc_hi8.as<uint8_t>(), T.yenc_lo8.as<uint8_t>(),
+                                   (int64_t) tt * 16 * TILE_ELEMS, lo_x, f8_x);
                     D.seg[0].mt_stride = (int64_t) VT * 16 * TILE_ELEMS; D.seg[0].nkt = 16;
                 }
                 if (t > 0) {
-                    D.seg[1].hi = y_hi + ((int64_t) tp * 16 + d * 8) * TILE_ELEMS; D.seg[1].lo = y_lo + ((int64_t) tp * 16 + d * 8) * TILE_ELEMS;
+                    D.seg[1] = seg(y_hi, y_lo, y_hi8, y_lo8, ((int64_t) tp * 16 + d * 8) * TILE_ELEMS, lo_h, f8_h);
                     D.seg[1].mt_stride = (int64_t) VT * 16 * TILE_ELEMS; D.seg[1].nkt = 8;
                 }
                 D.w_hi = W.w_hi.as<bf16>(); D.w_lo = W.w_lo.as<bf16>(); D.w_nkt = W.nkt_x + W.nkt_h;
+                D.w8_hi = W.w8_hi.as<uint8_t>(); D.w8_lo = W.w8_lo.as<uint8_t>(); D.acc_scale = W.acc_scale;
                 D.bias = (layer == 0 ? N->enc[d] : N->dec[d]).bias.as<float>();
                 D.c = T.c.as<float>() + (int64_t) d * VH * Bp;
-                D.y_hi = y_hi; D.y_lo = y_lo; D.y_mt_stride = (int64_t) VT * 16 * TILE_ELEMS; D.y_kt0 = tt * 16 + d * 8;
+                D.y_hi = y_hi; D.y_lo = y_lo; D.y_hi8 = y_hi8; D.y_lo8 = y_lo8;
+                D.y_mt_stride = (int64_t) VT * 16 * TILE_ELEMS; D.y_kt0 = tt * 16 + d * 8;
                 if (layer == 1 && d_hidden_dbg) { D.y_f32 = d_hidden_dbg + (int64_t) tt * 512 + d * VH; D.ldy = (int64_t) VT * 512; }
                 A.d[d] = D;
             }
@@ -183,17 +276,25 @@ int variant_forward_tc(pb_variant_net *N, const int8_t *d_images, int64_t B, flo
         Args A;
         A.M = (int) B; A.N = 512; A.c_ld = 0;
         Dir D = empty_dir();
+        const int slot = i == 0 ? 3 : 4, lo = (T.lo_mask >> slot) & 1, f8 = (T.f8_mask >> slot) & 1;
         if (i == 0) {
-            D.seg[0].hi = T.ydec_hi.as<bf16>(); D.seg[0].lo = ((T.lo_mask >> 3) & 1) ? T.ydec_lo.as<bf16>() : nullptr;
+            D.seg[0] = seg(T.ydec_hi.as<bf16>(), T.ydec_lo.as<bf16>(), T.ydec_hi8.as<uint8_t>(), T.ydec_lo8.as<uint8_t>(), 0, lo, f8);
             D.seg[0].mt_stride = (int64_t) VT * 16 * TILE_ELEMS; D.seg[0].nkt = VT * 16;
         } else {
-            D.seg[0].hi = T.act_hi[(i - 1) & 1].as<bf16>(); D.seg[0].lo = ((T.lo_mask >> 4) & 1) ? T.act_lo[(i - 1) & 1].as<bf16>() : nullptr;
+            const int a = (i - 1) & 1;
+            D.seg[0] = seg(T.act_hi[a].as<bf16>(), T.act_lo[a].as<bf16>(), T.act_hi8[a].as<uint8_t>(), T.act_lo8[a].as<uint8_t>(), 0, lo, f8);
             D.seg[0].mt_stride = (int64_t) 16 * TILE_ELEMS; D.seg[0].nkt = 16;
         }
         D.w_hi = T.lin[i].w_hi.as<bf16>(); D.w_lo = T.lin[i].w_lo.as<bf16>(); D.w_nkt = T.lin[i].nkt;
+        D.w8_hi = T.lin[i].w8_hi.as<uint8_t>(); D.w8_lo = T.lin[i].w8_lo.as<uint8_t>(); D.acc_scale = T.lin[i].acc_scale;
         D.bias = N->lin[i].bias.as<float>();
-        D.y_hi = T.act_hi[i & 1].as<bf16>(); D.y_lo = T.act_lo[i & 1].as<bf16>(); D.y_mt_stride = (int64_t) 16 * TILE_ELEMS; D.y_kt0 = 0;
-        if (i == 4) { D.y_f32 = T.final_f32.as<float>(); D.ldy = 512; }
+        if (i < 4) {             // linear_5 feeds only the fp32 copy read by the output layer
+            D.y_hi = T.act_hi[i & 1].as<bf16>(); D.y_lo = pick16(act_out.lo16, T.act_lo[i & 1]);
+            D.y_hi8 = pick8(act_out.hi8, T.act_hi8[i & 1]); D.y_lo8 = pick8(act_out.lo8, T.act_lo8[i & 1]);
+            D.y_mt_stride = (int64_t) 16 * TILE_ELEMS; D.y_kt0 = 0;
+        } else {
+            D.y_f32 = T.final_f32.as<float>(); D.ldy = 512;
+        }
         A.d[0] = D; A.d[1] = D;
         PB_TRY(launch_tc<tc::EPI_SELU>(A, (int) Mt, 4, 1, st));
         N->launches++;
@@ -362,25 +463,34 @@ int polish_forward_tc(pb_polish_net *N, const uint8_t *d_images, int64_t B, int6
 
 // ------------------------------------------------------------------------------------------------- self test
 // C[M][N] = A[M][K] W[N][K]^T + bias through the tcgen05 kernel (EPI_BIAS, fp32 output).  N % 256 == 0, K % 32 == 0.
-extern "C" int pb_test_tc_gemm(int M, int N, int K, const float *h_A, const float *h_W, const float *h_bias, float *h_out) {
+// variant_images = false: unscaled fp16 images, three products.  true: the variant network's images (tc_upload_lin with_f8),
+// a_lo x w_hi where `lo`, corrections in e4m3 where `f8`.
+static int test_tc_gemm(int M, int N, int K, const float *h_A, const float *h_W, const float *h_bias, float *h_out, bool variant_images, int lo, int f8) {
     if (N % 256 || K % 32 || M <= 0) { set_error("pb_test_tc_gemm: N %% 256 and K %% 32 must be 0"); return PB_ERR_ARG; }
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { set_error("no CUDA device: libpepper_b200 has no CPU fallback"); return PB_ERR_CUDA; }
     const int64_t Mt = ceil_div(M, 128);
-    std::vector<uint16_t> ahi, alo, whi, wlo;
-    tile_matrix(h_A, M, K, Mt * 128, K, ahi, alo);
-    tile_matrix(h_W, N, K, N, K, whi, wlo, 256);
-    DevBuf dahi, dalo, dwhi, dwlo, dbias, dout;
+    std::vector<uint16_t> ahi, alo;
+    F8Tiles a8{{}, {}, 1.f, tc::F8_LO_SCALE};
+    tile_matrix(h_A, M, K, Mt * 128, K, ahi, alo, 128, 1.f, &a8);
+    TcLin W;
+    DevBuf dahi, dalo, da8hi, da8lo, dbias, dout;
     PB_TRY(upload_tiles(dahi, dalo, ahi, alo));
-    PB_TRY(upload_tiles(dwhi, dwlo, whi, wlo));
+    PB_TRY(upload_f8(da8hi, da8lo, a8));
+    PB_TRY(upload_weight(h_W, N, K, N, K, variant_images, W.w_hi, W.w_lo, W.w8_hi, W.w8_lo, W.acc_scale));
     PB_TRY(dbias.reserve(sizeof(float) * N));
     PB_TRY(dout.reserve(sizeof(float) * (size_t) M * N));
     PB_CUDA(cudaMemcpy(dbias.p, h_bias, sizeof(float) * N, cudaMemcpyHostToDevice));
     Args A;
     A.M = M; A.N = N; A.c_ld = 0;
     Dir D = empty_dir();
-    D.seg[0].hi = dahi.as<bf16>(); D.seg[0].lo = dalo.as<bf16>(); D.seg[0].mt_stride = (int64_t) (K / 32) * TILE_ELEMS; D.seg[0].nkt = K / 32;
-    D.w_hi = dwhi.as<bf16>(); D.w_lo = dwlo.as<bf16>(); D.w_nkt = K / 32;
+    Seg &S = D.seg[0];
+    S.hi = dahi.as<bf16>();
+    if (variant_images && f8) { S.hi8 = da8hi.as<uint8_t>(); S.lo8 = lo ? da8lo.as<uint8_t>() : nullptr; }
+    else S.lo = (!variant_images || lo) ? dalo.as<bf16>() : nullptr;
+    S.mt_stride = (int64_t) (K / 32) * TILE_ELEMS; S.nkt = K / 32;
+    D.w_hi = W.w_hi.as<bf16>(); D.w_lo = W.w_lo.as<bf16>(); D.w8_hi = W.w8_hi.as<uint8_t>(); D.w8_lo = W.w8_lo.as<uint8_t>();
+    D.acc_scale = W.acc_scale; D.w_nkt = K / 32;
     D.bias = dbias.as<float>();
     D.y_f32 = dout.as<float>(); D.ldy = N;
     A.d[0] = D; A.d[1] = D;
@@ -388,7 +498,13 @@ extern "C" int pb_test_tc_gemm(int M, int N, int K, const float *h_A, const floa
     PB_CUDA(cudaGetLastError());
     PB_CUDA(cudaDeviceSynchronize());
     PB_CUDA(cudaMemcpy(h_out, dout.p, sizeof(float) * (size_t) M * N, cudaMemcpyDeviceToHost));
-    DevBuf *bufs[] = {&dahi, &dalo, &dwhi, &dwlo, &dbias, &dout};
+    DevBuf *bufs[] = {&dahi, &dalo, &da8hi, &da8lo, &W.w_hi, &W.w_lo, &W.w8_hi, &W.w8_lo, &dbias, &dout};
     for (auto *b : bufs) b->release();
     return PB_OK;
+}
+extern "C" int pb_test_tc_gemm(int M, int N, int K, const float *h_A, const float *h_W, const float *h_bias, float *h_out) {
+    return test_tc_gemm(M, N, K, h_A, h_W, h_bias, h_out, false, 1, 0);
+}
+extern "C" int pb_test_tc_gemm_f8(int M, int N, int K, const float *h_A, const float *h_W, const float *h_bias, float *h_out, int lo, int f8) {
+    return test_tc_gemm(M, N, K, h_A, h_W, h_bias, h_out, true, lo, f8);
 }

@@ -13,10 +13,16 @@
 // epilogue warps read the accumulator with tcgen05.ld (one TMEM lane = one batch row per thread), apply bias + cell,
 // and write the NEXT operand (h_t as bf16 hi/lo tiles) straight from registers, so activations never exist in fp32
 // in HBM between layers.
+//
+// The variant network's persistent kernels (k_tc_gemm_p, k_lstm_layer) can also run the two correction products of a k-tile
+// in e4m3 (tcgen05.mma kind::f8f6f4, one K32 MMA = half the tensor time of the two K16 fp16 MMAs it replaces): the main
+// product a_hi * w_hi stays fp16 and the corrections, ~2^-12 of it, only need a few significant bits.  See "e4m3 correction
+// operands" below.
 #pragma once
 #include "common.cuh"
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
+#include <cuda_fp8.h>
 
 namespace pb {
 namespace tc {
@@ -50,18 +56,22 @@ enum { EPI_BIAS = 0, EPI_SELU = 1, EPI_LSTM = 2, EPI_GRU = 3 };
 
 struct Seg {                       // one K-segment of the A operand
     const op_t *hi, *lo;  // lo == nullptr: exactly representable operand (int8 images), a_lo*w_hi product skipped
+    const uint8_t *hi8, *lo8;      // k_tc_gemm_p: hi8 != nullptr runs the corrections in e4m3 (lo8 == nullptr: without a_lo*w_hi)
     int64_t mt_stride;             // elements between consecutive row tiles
     int nkt;                       // k-tiles in this segment
 };
 struct Dir {
     Seg seg[2];
     const op_t *w_hi, *w_lo;   // [n_tile][w_nkt][TILE_ELEMS]
+    const uint8_t *w8_hi, *w8_lo;       // e4m3 weight images, same tiling (k_tc_gemm_p)
+    float acc_scale;                    // accumulator -> GEMM value (2^(E-12) for scaled weight images, else 1)
     int w_nkt;                          // k-tiles per n-tile of the packed weight (>= k-tiles of this launch)
     const float *bias;                  // [N]
     float *c;                           // LSTM cell state [H][c_ld]
     const op_t *hp_hi, *hp_lo; // GRU: previous hidden state as a tiled operand (k-tile = unit/32)
     int64_t hp_mt_stride;
-    op_t *y_hi, *y_lo;         // output operand tiles: tile (mt, y_kt0 + col/32)
+    op_t *y_hi, *y_lo;         // output operand tiles: tile (mt, y_kt0 + col/32); y_lo may be nullptr (k_tc_gemm_p)
+    uint8_t *y_hi8, *y_lo8;    // optional e4m3 output images (k_tc_gemm_p)
     int64_t y_mt_stride;
     int y_kt0;
     float *y_f32; int64_t ldy;          // optional fp32 copy  y_f32[row*ldy + col]
@@ -184,6 +194,106 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 
+// ---------------------------------------------------------------- e4m3 correction operands
+// A weight tensor w gets a power-of-two scale 2^-E with max|w * 2^-E| in [0.5, 1) (w' = w * 2^-E).  Its fp16 images hold
+// w'_hi * 2^12 and w'_lo * 2^12, its e4m3 images w'_hi and w'_lo * 2^12.  An activation a is fed as fp16 a_hi, e4m3(a) and
+// e4m3(a_lo * 2^12).  Then a_hi*w_hi (fp16), e4m3(a)*e4m3(w_lo) and e4m3(a_lo)*e4m3(w_hi) all land in the fp32 accumulator
+// at the same scale 2^(12-E), which the epilogue undoes exactly (Dir::acc_scale = 2^(E-12)).  The corrections carry e4m3's
+// 2^-4 relative rounding on terms ~2^-12 of the product: ~2^-16 relative, below the fp16 split's own error.
+//
+// 8-bit operand tiles use the same K-major no-swizzle canonical layout with 16-byte core-matrix rows: for a tile of R rows
+// x 32 k, element (r, k) sits at (k/16)*(R*16) + r*16 + k%16 — R*32 bytes, so the tile index arithmetic of the 16-bit
+// images (TILE_ELEMS / WTILE_ELEMS elements per tile) carries over unchanged with a byte pointer.  One K32 MMA covers a
+// k-tile; LBO (2048 B / 4096 B) and SBO (128 B) are the values of the 16-bit descriptors.
+constexpr int TILE8_BYTES = TILE_ELEMS;               // 4 KB: 128 rows x 32 k
+constexpr int WTILE8_BYTES = WTILE_ELEMS;             // 8 KB: 256 rows x 32 k
+constexpr float F8_LO_SCALE = 4096.f;                 // 2^12
+// Stage layout.  fp16 k-tile: A_hi | A_lo | W_hi | W_lo.  e4m3-correction k-tile: A_hi | A8_hi A8_lo | W_hi | W8_hi W8_lo
+// (A8_lo / W8_hi only when the a_lo*w_hi product runs).  A_hi and W_hi sit at the same offset in both.
+constexpr uint32_t ST_A_HI = 0, ST_A_LO = TILE_BYTES, ST_W_HI = 2 * TILE_BYTES, ST_W_LO = 2 * TILE_BYTES + WTILE_BYTES;
+constexpr uint32_t ST_A8_HI = TILE_BYTES, ST_A8_LO = TILE_BYTES + TILE8_BYTES;
+constexpr uint32_t ST_W8_HI = 2 * TILE_BYTES + WTILE_BYTES, ST_W8_LO = ST_W8_HI + WTILE8_BYTES;
+static_assert(ST_A8_LO + TILE8_BYTES <= ST_W_HI && ST_W8_LO + WTILE8_BYTES <= PSTAGE_BYTES, "e4m3 stage layout");
+// kind::f8f6f4, A = B = E4M3 (format 0), D = F32, both K-major, M = 128, N = 256
+constexpr uint32_t IDESC256_F8 = (1u << 4) | (0u << 7) | (0u << 10) | ((uint32_t) (PBN >> 3) << 17) | ((uint32_t) (BM >> 4) << 24);
+
+__host__ __device__ __forceinline__ uint8_t f8_bits(float v) { return (uint8_t) __nv_cvt_float_to_fp8(v, __NV_SATFINITE, __NV_E4M3); }
+__device__ __forceinline__ uint32_t f8x2(float a, float b) { return (uint32_t) __nv_cvt_float2_to_fp8x2(make_float2(a, b), __NV_SATFINITE, __NV_E4M3); }
+
+__device__ __forceinline__ void tc_mma_f8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, {%5, %6, %7, %8}, p;\n\t}"
+        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(0u), "r"(0u), "r"(0u), "r"(0u) : "memory");
+}
+
+// One k-tile into stage `st`.  a8_hi != nullptr selects the e4m3-correction layout; a_lo / a8_lo == nullptr skips the a_lo*w_hi
+// product (and, in e4m3 mode, the w8_hi tile it needs).
+__device__ __forceinline__ void load_ktile(uint32_t st, uint32_t bar, const op_t *a_hi, const op_t *a_lo, const uint8_t *a8_hi,
+                                           const uint8_t *a8_lo, const op_t *w_hi, const op_t *w_lo, const uint8_t *w8_hi,
+                                           const uint8_t *w8_lo) {
+    if (a8_hi) {
+        mbar_expect_tx(bar, TILE_BYTES + WTILE_BYTES + TILE8_BYTES + WTILE8_BYTES + (a8_lo ? TILE8_BYTES + WTILE8_BYTES : 0u));
+        bulk_g2s(st + ST_A_HI, a_hi, TILE_BYTES, bar);
+        bulk_g2s(st + ST_A8_HI, a8_hi, TILE8_BYTES, bar);
+        if (a8_lo) {
+            bulk_g2s(st + ST_A8_LO, a8_lo, TILE8_BYTES, bar);
+            bulk_g2s(st + ST_W8_HI, w8_hi, WTILE8_BYTES, bar);
+        }
+        bulk_g2s(st + ST_W_HI, w_hi, WTILE_BYTES, bar);
+        bulk_g2s(st + ST_W8_LO, w8_lo, WTILE8_BYTES, bar);
+    } else {
+        mbar_expect_tx(bar, (a_lo ? 2u : 1u) * TILE_BYTES + 2u * WTILE_BYTES);
+        bulk_g2s(st + ST_A_HI, a_hi, TILE_BYTES, bar);
+        if (a_lo) bulk_g2s(st + ST_A_LO, a_lo, TILE_BYTES, bar);
+        bulk_g2s(st + ST_W_HI, w_hi, WTILE_BYTES, bar);
+        bulk_g2s(st + ST_W_LO, w_lo, WTILE_BYTES, bar);
+    }
+}
+// The products of one k-tile in stage `st` (layout as load_ktile): fp16 a_hi*w_hi, then a_hi*w_lo (+ a_lo*w_hi) in fp16 or e4m3.
+__device__ __forceinline__ void mma_ktile(uint32_t tacc, uint32_t st, bool first, bool f8, bool has_lo) {
+#pragma unroll
+    for (int ks = 0; ks < BK / 16; ks++) {
+        const uint64_t a_hi = smem_desc_lbo(st + ST_A_HI + ks * 4096, 2048), b_hi = smem_desc_lbo(st + ST_W_HI + ks * 8192, 4096);
+        tc_mma(tacc, a_hi, b_hi, IDESC256, (!first || ks > 0) ? 1u : 0u);
+        if (!f8) {
+            tc_mma(tacc, a_hi, smem_desc_lbo(st + ST_W_LO + ks * 8192, 4096), IDESC256, 1u);
+            if (has_lo) tc_mma(tacc, smem_desc_lbo(st + ST_A_LO + ks * 4096, 2048), b_hi, IDESC256, 1u);
+        }
+    }
+    if (f8) {
+        tc_mma_f8(tacc, smem_desc_lbo(st + ST_A8_HI, 2048), smem_desc_lbo(st + ST_W8_LO, 4096), IDESC256_F8, 1u);
+        if (has_lo) tc_mma_f8(tacc, smem_desc_lbo(st + ST_A8_LO, 2048), smem_desc_lbo(st + ST_W8_HI, 4096), IDESC256_F8, 1u);
+    }
+}
+
+// 8 consecutive k (k0 % 8 == 0) of one row of the output operand at tile offset `tile` (elements / bytes): fp16 hi always,
+// fp16 lo / e4m3 hi / e4m3 lo where the pointer is set (only the images some consumer GEMM reads are written).
+__device__ __forceinline__ void put_op8(const float (&v)[8], op_t *hi, op_t *lo, uint8_t *hi8, uint8_t *lo8, int64_t tile, int k0, int r128) {
+    uint32_t h[4], l[4];
+    float res[8];
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        const uint16_t h0 = op_bits(v[2 * i]), h1 = op_bits(v[2 * i + 1]);
+        res[2 * i] = v[2 * i] - op_val(h0);
+        res[2 * i + 1] = v[2 * i + 1] - op_val(h1);
+        h[i] = (uint32_t) h0 | ((uint32_t) h1 << 16);
+        l[i] = (uint32_t) op_bits(res[2 * i]) | ((uint32_t) op_bits(res[2 * i + 1]) << 16);
+    }
+    const int64_t o = tile + (k0 >> 3) * 1024 + r128 * 8;
+    *reinterpret_cast<uint4 *>(hi + o) = make_uint4(h[0], h[1], h[2], h[3]);
+    if (lo) *reinterpret_cast<uint4 *>(lo + o) = make_uint4(l[0], l[1], l[2], l[3]);
+    const int64_t o8 = tile + (k0 >> 4) * 2048 + r128 * 16 + (k0 & 15);
+    if (hi8)
+        *reinterpret_cast<uint2 *>(hi8 + o8) = make_uint2(f8x2(v[0], v[1]) | (f8x2(v[2], v[3]) << 16), f8x2(v[4], v[5]) | (f8x2(v[6], v[7]) << 16));
+    if (lo8) {
+        float s[8];
+#pragma unroll
+        for (int i = 0; i < 8; i++) s[i] = res[i] * F8_LO_SCALE;
+        *reinterpret_cast<uint2 *>(lo8 + o8) = make_uint2(f8x2(s[0], s[1]) | (f8x2(s[2], s[3]) << 16), f8x2(s[4], s[5]) | (f8x2(s[6], s[7]) << 16));
+    }
+}
+
 template <int EPI>
 __global__ void __launch_bounds__(PG_THREADS, 1) k_tc_gemm_p(Args G, int n_mt, int n_nt /* 256-column tiles */, int n_dir) {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -230,13 +340,10 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_tc_gemm_p(Args G, int n_mt, i
                     mbar_wait(bar_empty + 8 * s, ph ^ 1u);
                     const Seg &S = (kt < nkt0) ? D.seg[0] : D.seg[1];
                     const int64_t off = (int64_t) mt * S.mt_stride + (int64_t) ((kt < nkt0) ? kt : kt - nkt0) * TILE_ELEMS;
-                    const uint32_t st = smem_base + s * PSTAGE_BYTES;
-                    mbar_expect_tx(bar_full + 8 * s, (S.lo ? 2u : 1u) * TILE_BYTES + 2u * WTILE_BYTES);
-                    bulk_g2s(st, S.hi + off, TILE_BYTES, bar_full + 8 * s);
-                    if (S.lo) bulk_g2s(st + TILE_BYTES, S.lo + off, TILE_BYTES, bar_full + 8 * s);
                     const int64_t woff = ((int64_t) nt * D.w_nkt + kt) * WTILE_ELEMS;
-                    bulk_g2s(st + 2 * TILE_BYTES, D.w_hi + woff, WTILE_BYTES, bar_full + 8 * s);
-                    bulk_g2s(st + 2 * TILE_BYTES + WTILE_BYTES, D.w_lo + woff, WTILE_BYTES, bar_full + 8 * s);
+                    load_ktile(smem_base + s * PSTAGE_BYTES, bar_full + 8 * s, S.hi + off, S.lo ? S.lo + off : nullptr,
+                               S.hi8 ? S.hi8 + off : nullptr, S.lo8 ? S.lo8 + off : nullptr, D.w_hi + woff, D.w_lo + woff,
+                               D.w8_hi ? D.w8_hi + woff : nullptr, D.w8_lo ? D.w8_lo + woff : nullptr);
                 }
             }
         }
@@ -256,17 +363,9 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_tc_gemm_p(Args G, int n_mt, i
                     const uint32_t s = g % PSTAGES, ph = (g / PSTAGES) & 1u;
                     mbar_wait(bar_full + 8 * s, ph);
                     tc_fence_after();
-                    const bool has_lo = ((kt < nkt0) ? D.seg[0].lo : D.seg[1].lo) != nullptr;
-                    const uint32_t st = smem_base + s * PSTAGE_BYTES;
-#pragma unroll
-                    for (int ks = 0; ks < BK / 16; ks++) {
-                        const uint64_t a_hi = smem_desc_lbo(st + ks * 4096, 2048), a_lo = smem_desc_lbo(st + TILE_BYTES + ks * 4096, 2048);
-                        const uint64_t b_hi = smem_desc_lbo(st + 2 * TILE_BYTES + ks * 8192, 4096);
-                        const uint64_t b_lo = smem_desc_lbo(st + 2 * TILE_BYTES + WTILE_BYTES + ks * 8192, 4096);
-                        tc_mma(tacc, a_hi, b_hi, IDESC256, (kt > 0 || ks > 0) ? 1u : 0u);
-                        tc_mma(tacc, a_hi, b_lo, IDESC256, 1u);
-                        if (has_lo) tc_mma(tacc, a_lo, b_hi, IDESC256, 1u);
-                    }
+                    const Seg &S = (kt < nkt0) ? D.seg[0] : D.seg[1];
+                    const bool f8 = S.hi8 != nullptr;
+                    mma_ktile(tacc, smem_base + s * PSTAGE_BYTES, kt == 0, f8, (f8 ? (const void *) S.lo8 : (const void *) S.lo) != nullptr);
                     tc_commit(bar_empty + 8 * s);
                 }
                 tc_commit(bar_accf + 8 * buf);
@@ -325,17 +424,13 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_tc_gemm_p(Args G, int n_mt, i
                         float v[8];
 #pragma unroll
                         for (int i = 0; i < 8; i++) {
-                            const float x = __uint_as_float(acc[g8 * 8 + i]) + __ldg(D.bias + col0 + g8 * 8 + i);
+                            const float x = __uint_as_float(acc[g8 * 8 + i]) * D.acc_scale + __ldg(D.bias + col0 + g8 * 8 + i);
                             v[i] = (EPI == EPI_SELU) ? selu(x) : x;
                         }
                         if (valid) {
-                            if (D.y_hi) {
-                                uint4 hi, lo;
-                                split8(v, hi, lo);
-                                const int64_t o = (int64_t) mt * D.y_mt_stride + (int64_t) (D.y_kt0 + col0 / 32) * TILE_ELEMS + g8 * 1024 + r128 * 8;
-                                *reinterpret_cast<uint4 *>(D.y_hi + o) = hi;
-                                *reinterpret_cast<uint4 *>(D.y_lo + o) = lo;
-                            }
+                            if (D.y_hi)
+                                put_op8(v, D.y_hi, D.y_lo, D.y_hi8, D.y_lo8, (int64_t) mt * D.y_mt_stride + (int64_t) (D.y_kt0 + col0 / 32) * TILE_ELEMS,
+                                        g8 * 8, r128);
                             if (D.y_f32) {
                                 float4 *dst = reinterpret_cast<float4 *>(D.y_f32 + (int64_t) row * D.ldy + col0 + g8 * 8);
                                 dst[0] = make_float4(v[0], v[1], v[2], v[3]);
@@ -349,8 +444,9 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_tc_gemm_p(Args G, int n_mt, i
 #pragma unroll
                     for (int u = 0; u < 8; u++) {
                         const float4 bz = __ldg(reinterpret_cast<const float4 *>(D.bias + col0 + 4 * u));
-                        const float v0 = __uint_as_float(acc[4 * u + 0]) + bz.x, v1 = __uint_as_float(acc[4 * u + 1]) + bz.y;
-                        const float v2 = __uint_as_float(acc[4 * u + 2]) + bz.z, v3 = __uint_as_float(acc[4 * u + 3]) + bz.w;
+                        const float sc = D.acc_scale;
+                        const float v0 = __uint_as_float(acc[4 * u + 0]) * sc + bz.x, v1 = __uint_as_float(acc[4 * u + 1]) * sc + bz.y;
+                        const float v2 = __uint_as_float(acc[4 * u + 2]) * sc + bz.z, v3 = __uint_as_float(acc[4 * u + 3]) * sc + bz.w;
                         if (EPI == EPI_LSTM) {
                             const float ig = sigm(v0), fg = sigm(v1), gg = tanh_fast(v2), og = sigm(v3);
                             const float cn = fg * st[cl * 8 + u] + ig * gg;
@@ -363,11 +459,8 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_tc_gemm_p(Args G, int n_mt, i
                         }
                     }
                     if (valid) {
-                        uint4 hi, lo;
-                        split8(hn, hi, lo);
-                        const int64_t o = (int64_t) mt * D.y_mt_stride + (int64_t) (D.y_kt0 + (j0 >> 5)) * TILE_ELEMS + ((j0 & 31) >> 3) * 1024 + r128 * 8;
-                        *reinterpret_cast<uint4 *>(D.y_hi + o) = hi;
-                        *reinterpret_cast<uint4 *>(D.y_lo + o) = lo;
+                        put_op8(hn, D.y_hi, D.y_lo, D.y_hi8, D.y_lo8, (int64_t) mt * D.y_mt_stride + (int64_t) (D.y_kt0 + (j0 >> 5)) * TILE_ELEMS,
+                                j0 & 31, r128);
                         if (D.y_f32) {
                             float4 *dst = reinterpret_cast<float4 *>(D.y_f32 + (int64_t) row * D.ldy + j0);
                             dst[0] = make_float4(hn[0], hn[1], hn[2], hn[3]);
@@ -400,18 +493,23 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_tc_gemm_p(Args G, int n_mt, i
 // launches, prologues and tails than the per-step kernel above (kept as the cross-check path).
 struct LstmLayer {
     const op_t *x_hi, *x_lo;           // input sequence operand: tile (mt, t, kt) at mt * x_mt_stride + (t * x_nkt + kt) * TILE_ELEMS
+    const uint8_t *x_hi8, *x_lo8;      // its e4m3 images (same tile offsets, bytes)
     int64_t x_mt_stride;
     int x_nkt;
     const op_t *w_hi[2], *w_lo[2];     // per direction: [4 n-tiles][x_nkt + 8][WTILE_ELEMS]
+    const uint8_t *w8_hi[2], *w8_lo[2];
+    float acc_scale[2];                // accumulator -> gate pre-activation (2^(E-12) of the direction's weight scale)
     const float *bias[2];
     float *c[2];                                // cell state per direction [256][c_ld], zero initialised
     op_t *y_hi, *y_lo;                 // output sequence operand [mt][T][16] tiles; (time tt, direction d) -> k-tiles tt * 16 + d * 8 ...
+    uint8_t *y_hi8, *y_lo8;            // its e4m3 images; y_lo / y_hi8 / y_lo8 == nullptr: not written (no consumer reads it)
     int64_t y_mt_stride;
     float *y_f32;                               // optional fp32 copy [row][T][512]
     int64_t ldy;
     int M, n_mt, T;
     int64_t c_ld;
     int lo_x, lo_h;                             // 1: the a_lo x w_hi product of the x-part / h-part is executed (0: two products)
+    int f8_x, f8_h;                             // 1: the corrections of the x-part / h-part run in e4m3
 };
 
 __global__ void __launch_bounds__(PG_THREADS, 1) k_lstm_layer(LstmLayer G) {
@@ -451,10 +549,13 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_lstm_layer(LstmLayer G) {
                     for (int kt = 0; kt < nkt; kt++, g++) {
                         const uint32_t s = g % PSTAGES, ph = (g / PSTAGES) & 1u;
                         mbar_wait(bar_empty + 8 * s, ph ^ 1u);
-                        const op_t *a_hi, *a_lo;
+                        const op_t *a_hi, *a_lo = nullptr;
+                        const uint8_t *a8_hi = nullptr, *a8_lo = nullptr;
                         if (kt < G.x_nkt) {
                             const int64_t off = (int64_t) mt * G.x_mt_stride + ((int64_t) tt * G.x_nkt + kt) * TILE_ELEMS;
-                            a_hi = G.x_hi + off; a_lo = (G.x_lo && G.lo_x) ? G.x_lo + off : nullptr;
+                            a_hi = G.x_hi + off;
+                            if (G.f8_x) { a8_hi = G.x_hi8 + off; if (G.lo_x) a8_lo = G.x_lo8 + off; }
+                            else if (G.lo_x) a_lo = G.x_lo + off;
                         } else {
                             const int kk = kt - G.x_nkt;
                             if (kk == 0 && nt == 0) {
@@ -463,15 +564,13 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_lstm_layer(LstmLayer G) {
                                 asm volatile("fence.proxy.async;" ::: "memory");
                             }
                             const int64_t off = (int64_t) mt * G.y_mt_stride + ((int64_t) tp * 16 + dir * 8 + kk) * TILE_ELEMS;
-                            a_hi = G.y_hi + off; a_lo = G.lo_h ? G.y_lo + off : nullptr;
+                            a_hi = G.y_hi + off;
+                            if (G.f8_h) { a8_hi = G.y_hi8 + off; if (G.lo_h) a8_lo = G.y_lo8 + off; }
+                            else if (G.lo_h) a_lo = G.y_lo + off;
                         }
-                        const uint32_t st = smem_base + s * PSTAGE_BYTES;
-                        mbar_expect_tx(bar_full + 8 * s, (a_lo ? 2u : 1u) * TILE_BYTES + 2u * WTILE_BYTES);
-                        bulk_g2s(st, a_hi, TILE_BYTES, bar_full + 8 * s);
-                        if (a_lo) bulk_g2s(st + TILE_BYTES, a_lo, TILE_BYTES, bar_full + 8 * s);
                         const int64_t woff = ((int64_t) nt * w_nkt + kt) * WTILE_ELEMS;
-                        bulk_g2s(st + 2 * TILE_BYTES, G.w_hi[dir] + woff, WTILE_BYTES, bar_full + 8 * s);
-                        bulk_g2s(st + 2 * TILE_BYTES + WTILE_BYTES, G.w_lo[dir] + woff, WTILE_BYTES, bar_full + 8 * s);
+                        load_ktile(smem_base + s * PSTAGE_BYTES, bar_full + 8 * s, a_hi, a_lo, a8_hi, a8_lo, G.w_hi[dir] + woff,
+                                   G.w_lo[dir] + woff, G.w8_hi[dir] ? G.w8_hi[dir] + woff : nullptr, G.w8_lo[dir] ? G.w8_lo[dir] + woff : nullptr);
                     }
                 }
             }
@@ -490,17 +589,8 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_lstm_layer(LstmLayer G) {
                         const uint32_t s = g % PSTAGES, ph = (g / PSTAGES) & 1u;
                         mbar_wait(bar_full + 8 * s, ph);
                         tc_fence_after();
-                        const bool has_lo = kt >= G.x_nkt ? (G.lo_h != 0) : (G.x_lo != nullptr && G.lo_x != 0);
-                        const uint32_t st = smem_base + s * PSTAGE_BYTES;
-#pragma unroll
-                        for (int ks = 0; ks < BK / 16; ks++) {
-                            const uint64_t a_hi = smem_desc_lbo(st + ks * 4096, 2048), a_lo = smem_desc_lbo(st + TILE_BYTES + ks * 4096, 2048);
-                            const uint64_t b_hi = smem_desc_lbo(st + 2 * TILE_BYTES + ks * 8192, 4096);
-                            const uint64_t b_lo = smem_desc_lbo(st + 2 * TILE_BYTES + WTILE_BYTES + ks * 8192, 4096);
-                            tc_mma(tacc, a_hi, b_hi, IDESC256, (kt > 0 || ks > 0) ? 1u : 0u);
-                            tc_mma(tacc, a_hi, b_lo, IDESC256, 1u);
-                            if (has_lo) tc_mma(tacc, a_lo, b_hi, IDESC256, 1u);
-                        }
+                        const bool xpart = kt < G.x_nkt;
+                        mma_ktile(tacc, smem_base + s * PSTAGE_BYTES, kt == 0, (xpart ? G.f8_x : G.f8_h) != 0, (xpart ? G.lo_x : G.lo_h) != 0);
                         tc_commit(bar_empty + 8 * s);
                     }
                     tc_commit(bar_accf + 8 * buf);
@@ -515,6 +605,7 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_lstm_layer(LstmLayer G) {
         const bool valid = row < G.M;
         float *cst = G.c[dir];
         const float *bias = G.bias[dir];
+        const float sc = G.acc_scale[dir];
         uint32_t it = 0;
         for (int t = 0; t < G.T; t++) {
             const int tt = dir ? G.T - 1 - t : t;
@@ -543,19 +634,16 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_lstm_layer(LstmLayer G) {
 #pragma unroll
                     for (int u = 0; u < 8; u++) {
                         const float4 bz = __ldg(reinterpret_cast<const float4 *>(bias + col0 + 4 * u));
-                        const float v0 = __uint_as_float(acc[4 * u + 0]) + bz.x, v1 = __uint_as_float(acc[4 * u + 1]) + bz.y;
-                        const float v2 = __uint_as_float(acc[4 * u + 2]) + bz.z, v3 = __uint_as_float(acc[4 * u + 3]) + bz.w;
+                        const float v0 = __uint_as_float(acc[4 * u + 0]) * sc + bz.x, v1 = __uint_as_float(acc[4 * u + 1]) * sc + bz.y;
+                        const float v2 = __uint_as_float(acc[4 * u + 2]) * sc + bz.z, v3 = __uint_as_float(acc[4 * u + 3]) * sc + bz.w;
                         const float ig = sigm(v0), fg = sigm(v1), gg = tanh_fast(v2), og = sigm(v3);
                         const float cn = fg * st[cl * 8 + u] + ig * gg;
                         st[cl * 8 + u] = cn;
                         hn[u] = og * tanh_fast(cn);
                     }
                     if (valid) {
-                        uint4 hi, lo;
-                        split8(hn, hi, lo);
-                        const int64_t o = (int64_t) mt * G.y_mt_stride + (int64_t) (y_kt0 + (j0 >> 5)) * TILE_ELEMS + ((j0 & 31) >> 3) * 1024 + r128 * 8;
-                        *reinterpret_cast<uint4 *>(G.y_hi + o) = hi;
-                        *reinterpret_cast<uint4 *>(G.y_lo + o) = lo;
+                        put_op8(hn, G.y_hi, G.y_lo, G.y_hi8, G.y_lo8, (int64_t) mt * G.y_mt_stride + (int64_t) (y_kt0 + (j0 >> 5)) * TILE_ELEMS,
+                                j0 & 31, r128);
                         if (G.y_f32) {
                             float4 *dst = reinterpret_cast<float4 *>(G.y_f32 + (int64_t) row * G.ldy + (int64_t) tt * 512 + dir * 256 + j0);
                             dst[0] = make_float4(hn[0], hn[1], hn[2], hn[3]);
@@ -984,8 +1072,9 @@ __global__ void __launch_bounds__(PG_THREADS, 1) k_gru_layer(GruWin G) {
 }
 
 // ---------------------------------------------------------------- operand preparation kernels
-// int8 images [B][T][F] -> tiled operand [mt][T][1 k-tile] (hi only; |v| <= 128 is exact in bf16)
-__global__ void k_tc_pack_images(const int8_t *__restrict__ img, op_t *__restrict__ op, int64_t B, int T, int F) {
+// int8 images [B][T][F] -> tiled operand [mt][T][1 k-tile] (hi only; |v| <= 128 is exact in bf16), and when op8 is set its
+// e4m3 image (the a_hi operand of the a_hi*w_lo correction; e4m3 rounds |v| > 16 to 4 significant bits, ~2^-16 of the product)
+__global__ void k_tc_pack_images(const int8_t *__restrict__ img, op_t *__restrict__ op, uint8_t *__restrict__ op8, int64_t B, int T, int F) {
     const int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;     // one thread per (row, t, kc)
     const int64_t total = ceil_div(B, 128) * 128 * T * 4;
     if (i >= total) return;
@@ -993,17 +1082,20 @@ __global__ void k_tc_pack_images(const int8_t *__restrict__ img, op_t *__restric
     const int64_t rt = i >> 2;
     const int t = (int) (rt % T);
     const int64_t row = rt / T;
-    uint32_t w[4] = {0, 0, 0, 0};
-    if (row < B) {
+    float v[8];
 #pragma unroll
-        for (int e = 0; e < 8; e++) {
-            const int k = kc * 8 + e;
-            const float v = (k < F) ? (float) img[(row * T + t) * F + k] : 0.f;
-            w[e >> 1] |= (uint32_t) op_bits(v) << (16 * (e & 1));
-        }
+    for (int e = 0; e < 8; e++) {
+        const int k = kc * 8 + e;
+        v[e] = (row < B && k < F) ? (float) img[(row * T + t) * F + k] : 0.f;
     }
-    const int64_t o = ((row >> 7) * T + t) * TILE_ELEMS + kc * 1024 + (row & 127) * 8;
-    *reinterpret_cast<uint4 *>(op + o) = make_uint4(w[0], w[1], w[2], w[3]);
+    uint32_t w[4];
+#pragma unroll
+    for (int i = 0; i < 4; i++) w[i] = (uint32_t) op_bits(v[2 * i]) | ((uint32_t) op_bits(v[2 * i + 1]) << 16);
+    const int64_t tile = ((row >> 7) * T + t) * TILE_ELEMS;
+    *reinterpret_cast<uint4 *>(op + tile + kc * 1024 + (row & 127) * 8) = make_uint4(w[0], w[1], w[2], w[3]);
+    if (op8)
+        *reinterpret_cast<uint2 *>(op8 + tile + (kc >> 1) * 2048 + (row & 127) * 16 + (kc & 1) * 8) =
+            make_uint2(f8x2(v[0], v[1]) | (f8x2(v[2], v[3]) << 16), f8x2(v[4], v[5]) | (f8x2(v[6], v[7]) << 16));
 }
 
 }  // namespace tc

@@ -199,6 +199,12 @@ class VariantNet:
         self.L.pb_variant_net_set_lo_mask.argtypes = [C.c_void_p, C.c_int]
         _lib.check(self.L.pb_variant_net_set_lo_mask(self.h, mask), "pb_variant_net_set_lo_mask")
 
+    def set_f8_mask(self, mask: int) -> None:
+        """Bit set (same bits as set_lo_mask) = that GEMM runs its correction products (a_hi x w_lo, and a_lo x w_hi where the
+        lo mask keeps it) as e4m3 tensor-core MMAs next to the fp16 a_hi x w_hi.  Default 0x1f; 0 = the fp16 split everywhere."""
+        self.L.pb_variant_net_set_f8_mask.argtypes = [C.c_void_p, C.c_int]
+        _lib.check(self.L.pb_variant_net_set_f8_mask(self.h, mask), "pb_variant_net_set_f8_mask")
+
     def launches(self) -> int:
         n = C.c_int64(0)
         _lib.check(self.L.pb_variant_net_launches(self.h, C.byref(n)), "launches")

@@ -17,6 +17,43 @@ from pepper_b200 import weights  # noqa: E402
 from tests.test_nets_gpu import _variant_images, _polish_images  # noqa: E402
 
 out = {"variant": [], "polish": []}
+if len(sys.argv) > 1 and sys.argv[1] == "f8":
+    # `exp_products.py f8`: the variant net at the default lo_mask with each f8_mask choice — error against the oracle and the
+    # device time of every kernel of one 9,472-candidate chunk (torch.profiler, in launch order)
+    import torch
+    F8 = {0x1f: "every correction in e4m3 (default)", 0x00: "fp16 split everywhere", 0x1e: "encoder fp16, rest e4m3",
+          0x07: "LSTM layers e4m3, head fp16", 0x18: "head e4m3, LSTM layers fp16"}
+    big = _variant_images(9472, 11)
+    tnet = VariantNet(weights.random_variant_state(0))
+    for mask, name in F8.items():
+        row = {"f8_mask": mask, "what": name, "max_dh": 0.0, "max_dp": 0.0, "argmax_mismatch_outside_margin": 0, "n": 0}
+        for seed in (1, 2, 3):
+            state = nets.make_variant_weights(seed)
+            x = _variant_images(700, seed)
+            want, whid = nets.variant_predict(state, x, threads=16, return_hidden=True)
+            net = VariantNet(state)
+            net.set_f8_mask(mask)
+            got, hid = net.predict(x, return_hidden=True)
+            net.close()
+            srt = np.sort(want, axis=1)
+            clear = (srt[:, -1] - srt[:, -2]) > 1e-4
+            row["max_dh"] = max(row["max_dh"], float(np.abs(hid - whid).max()))
+            row["max_dp"] = max(row["max_dp"], float(np.abs(got - want).max()))
+            row["argmax_mismatch_outside_margin"] += int((got.argmax(1)[clear] != want.argmax(1)[clear]).sum())
+            row["n"] += int(clear.sum())
+        tnet.set_f8_mask(mask)
+        for _ in range(3):
+            tnet.predict(big)
+        with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+            tnet.predict(big)
+        ev = sorted((e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA and e.name.startswith(("void pb::tc::k_", "pb::tc::k_"))),
+                    key=lambda e: e.time_range.start)
+        row["kernel_ms_one_chunk"] = [[e.name.split("(")[0].replace("void ", ""), round(e.device_time / 1e3, 3)] for e in ev]
+        out["variant"].append(row)
+        print(json.dumps(row), file=sys.stderr, flush=True)
+    tnet.close()
+    print(json.dumps(out))
+    sys.exit(0)
 VN = {0x1f: "all x3", 0x1e: "encoder h x2", 0x1d: "decoder x x2", 0x1b: "decoder h x2", 0x17: "linear_1 x2", 0x0f: "linear_2-5 x2",
       0x1a: "encoder h + decoder h x2 (shipped default)", 0x18: "both LSTM layers x2, head x3", 0x07: "head x2, LSTM x3", 0x00: "all x2"}
 if len(sys.argv) > 1:                       # e.g. `exp_products.py 0x1f,0x1a`: only these variant masks, polish skipped
